@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: SPGNN-3 (st_pgat_spgnn_3) training step on synthetic airway-tree batches.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--trees B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--trees B] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one iteration of the reference's GCN_STEPS loop (job_runner.py:1892-1919) over one batch of B trees
@@ -248,6 +248,36 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
+DUMP_LOGIT_ROWS = 1 << 16
+
+
+def dump_outputs(out_dir, net, loss, logits):
+    """What the last timed train step left to its caller, as float32 .npy files (about 26 MB for the headline), so
+    that two builds run with the same arguments can be compared output for output:
+      loss.npy           the step's masked weighted cross-entropy (scalar)
+      logits_sample.npy  forward logits of DUMP_LOGIT_ROWS nodes drawn without replacement by numpy's default_rng(SEED),
+                         in ascending node order (the full [N, 22] tensor is 108 MB at 4096 trees)
+      params.npy         every parameter after the step's SGD update, flattened in net.parameters() order
+      grads.npy          the step's gradients in the same layout (zeros for a parameter without one)
+    Two runs of one build are not bit-identical: on a B200 (1000 W limit) the headline's loss matched exactly, the
+    logits to 5e-6 and the gradients to 8e-6 of their largest entry, so compare with a tolerance."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = logits.shape[0]
+    rows = np.sort(np.random.default_rng(SEED).choice(n, size=min(n, DUMP_LOGIT_ROWS), replace=False))
+    params = list(net.parameters())
+    arrays = {
+        "loss": loss.reshape(()),
+        "logits_sample": logits[torch.from_numpy(rows).to(logits.device)],
+        "params": torch.cat([p.detach().reshape(-1) for p in params]),
+        "grads": torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1)
+                            for p in params]),
+    }
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -295,6 +325,10 @@ def run_ours(args):
     for _ in range(args.warmup):
         step()
     barrier()
+    last = {}
+    hook = None
+    if args.dump_outputs and rank == 0:          # keeps a reference to each step's logits, no copy inside the timed loop
+        hook = net.register_forward_hook(lambda m, i, o: last.__setitem__("logits", o[0].detach()))
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
@@ -305,6 +339,9 @@ def run_ours(args):
         loss = step()
     e1.record()
     barrier()
+    if hook is not None:
+        hook.remove()
+        dump_outputs(args.dump_outputs, net, loss, last.pop("logits"))
     ms = e0.elapsed_time(e1) / args.steps
     launches = L.launch_count() - l0                     # this library's kernel launches inside the timed region
     clocks = sampler.stop() if sampler else None
@@ -562,7 +599,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-small", action="store_true", help="skip the 64-tree / single-scan latency leg")
     ap.add_argument("--gemm-mode", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last "
+                    "one computed (loss, a fixed sample of logits, updated parameters, gradients) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

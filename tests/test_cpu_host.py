@@ -31,8 +31,10 @@ def test_library_builds_loads_and_exports_every_header_symbol():
 
 def test_library_is_sm100a_with_lineinfo():
     import subprocess
+    from spgnn_b200 import build
     from spgnn_b200._lib import LIB_PATH
-    out = subprocess.run(["cuobjdump", "--list-elf", LIB_PATH], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")       # the toolkit the library was built with
+    out = subprocess.run([cuobjdump, "--list-elf", LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 
@@ -215,6 +217,31 @@ def test_bench_workloads_and_launch_list_summary():
     first = out.splitlines()[0]
     assert first.startswith("one training step: launches 109"), first
     assert "tn_planes_kernel" in out and "gat_tree_bwd_kernel" in out
+
+
+def test_bench_dump_outputs_at_headline_size(tmp_path):
+    """bench.py --dump-outputs: float32 arrays under 64 MB in all at the headline's shapes (4096 trees x 301 nodes),
+    the same logit rows every run; --steps 0 is refused rather than timing nothing."""
+    import subprocess
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    from spgnn_b200 import models as sm
+    model, _, method, _ = bench.workload(bench.HEADLINE)
+    net = getattr(sm, method.split(".")[-1])(**model)
+    logits = torch.arange(4096 * 301 * 22, dtype=torch.float32).reshape(-1, 22)
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(str(d), net, torch.tensor(1.5), logits)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["grads.npy", "logits_sample.npy", "loss.npy", "params.npy"]
+    arrays = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert all(a.dtype == np.float32 for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    assert arrays["params"].size == sum(p.numel() for p in net.parameters()) == arrays["grads"].size
+    assert arrays["logits_sample"].shape == (bench.DUMP_LOGIT_ROWS, 22) and float(arrays["loss"]) == 1.5
+    assert np.array_equal(arrays["logits_sample"], np.load(tmp_path / "b" / "logits_sample.npy"))
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert r.returncode != 0 and "--steps" in r.stderr
 
 
 def test_host_row_packer_round_trips_on_the_cpu():
