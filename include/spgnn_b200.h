@@ -344,18 +344,24 @@ int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp
                       void* ws, int64_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
- * Weighted-sum aggregation (DGL SpMM copy_u.sum with degree norms): GraphConv and GINConv-mean.
- *   out[v, :] = act( post[v] * sum_{s in seg(v)} pre[nbr[s]] * x[nbr[s], :] + self_coef * x[v, :] + bias )
- * pre/post/bias may be null; self_coef is read from device memory (GIN's 1+eps) when self_coef_ptr != null
- * (value = 1 + *self_coef_ptr), else 0.  Forward uses the in-CSC, backward the out-CSR with pre/post swapped.
- * Replaces GraphConv (models.py:172-182) and GINConv "mean" (models.py:358-383) message passing.
+ * Weighted-sum aggregation (DGL SpMM copy_u.sum with degree norms): GraphConv, GINConv-mean, SAGEConv mean / gcn.
+ *   out[v, :] = act( post[v] * (sum_{s in seg(v)} pre[nbr[s]] * x[nbr[s], :] + [self_in] pre[v] * x[v, :])
+ *                    + self_coef * x[v, :] + add[v, :] + bias )            for v < N
+ * The two self terms are read only for v < n_self (n_self <= N; on a sampled block the destination rows): self_in
+ * puts x[v] inside the norm (SAGEConv 'gcn': (sum + x[v]) / (deg + 1)), self_coef outside it (read from device
+ * memory, GIN's 1+eps, when self_coef_ptr != null, value = 1 + *self_coef_ptr; else 0).  pre/post/add/bias may be
+ * null.  Forward uses the in-CSC with N = destination rows, backward the out-CSR with pre/post swapped and N = source
+ * rows.  Replaces GraphConv (models.py:172-182), GINConv "mean" (models.py:358-383) and SAGEConv "mean" / "gcn"
+ * message passing.
  * ---------------------------------------------------------------------------------- */
 int spgnn_spmm(const float* x, int64_t ldx, const int32_t* ptr, const int32_t* nbr,
-               const float* pre, const float* post, const float* self_eps_ptr,
-               const float* bias, int act, float slope,
+               const float* pre, const float* post, const float* self_eps_ptr, int self_in, int64_t n_self,
+               const float* add, int64_t ld_add, const float* bias, int act, float slope,
                float* out, int64_t ldo, int64_t N, int64_t F, void* stream);
 /* deg^-1/2 and 1/deg (clamped at 1) from a ptr array: norm_sqrt[N], norm_inv[N] (either may be null) */
 int spgnn_degree_norms(const int32_t* ptr, int64_t N, float* norm_sqrt, float* norm_inv, void* stream);
+/* out[i] = 1 / max(deg(i) + add, 1) from a ptr array (SAGEConv mean: add 0, gcn: add 1) */
+int spgnn_inv_degree(const int32_t* ptr, int64_t N, float add, float* out, void* stream);
 
 /* SAGEConv "pool": neigh[v,f] = max_{u->v} m[u,f]; arg[v,f] = in-slot of the max (first max).
  * Backward: dm[u,f] = sum over out-edges (u->v, slot s) of g[v,f] * [arg[v,f] == s].
@@ -365,6 +371,40 @@ int spgnn_sage_maxpool_fwd(const float* m, int64_t ldm, const int32_t* in_ptr, c
 int spgnn_sage_maxpool_bwd(const float* g, int64_t ldg, const int32_t* arg,
                            const int32_t* out_ptr, const int32_t* out_dst, const int32_t* out_slot,
                            float* dm, int64_t lddm, int64_t N, int64_t F, void* stream);
+
+/* ------------------------------------------------------------------------------------
+ * SAGEConv "lstm" reducer (DGL 0.7 _lstm_reducer: nn.LSTM(D, D, batch_first=True) over each destination's in-edge
+ * messages in in-CSC order, zero initial state, h_T = the aggregate; gate order i, f, g, o).
+ * Rows are the destinations sorted by in-degree, descending and stable, so step t runs over the first n_t rows
+ * (n_t = #destinations with in-degree > t) and its rows are a contiguous block at row off_t = sum_{s<t} n_s of the
+ * per-step buffers (sum_t n_t = E).
+ *   lstm_order_count / _scatter : the stable counting sort.  key = max_deg - deg (so descending degree), chunk = 256
+ *       destinations; count writes counts[key * n_chunks + chunk] (int64), the caller scans them (spgnn_scan_i64)
+ *       into offs, scatter writes perm[row] = destination and rank[destination] = row.  max_deg < 12288.
+ *   lstm_cell_fwd (step t): pre = P[src(v, t)] + R[r] (R = H_{t-1}[:n_t] W_hh^T, null at t = 0), with P = X W_ih^T +
+ *       b_ih + b_hh [n_src, 4D]; c = f c_prev + i g, h = o tanh(c).  Saves the gate activations (fp32 stored as
+ *       their high / low 16-bit halves in the two planes of `gates`, the layout the backward overwrites with the
+ *       gate-gradient planes in place) and c.  Rows r < n_next continue: h goes as planes to `h_next` (row r), the
+ *       operand of step t+1's GEMM; the other rows end here: h goes to out[perm[r]] (fp32).
+ *   lstm_cell_bwd (step t): dh = r < n_next ? dh_rec[r] (= dgates_{t+1} W_hh) : g_out[perm[r]]; dc carried in
+ *       dc[r]; writes the pre-activation gradients as planes over the saved gates.
+ *   lstm_dp : dP[u] = sum over u's out-edges (u -> v, in-slot s) of dgates row off[s - in_ptr[v]] + rank[v]; a
+ *       deterministic gather over the out-CSR, no atomics.
+ * D % 4 == 0; planes row strides (ld) multiples of 8.
+ * ---------------------------------------------------------------------------------- */
+int spgnn_lstm_order_count(const int32_t* in_ptr, int64_t N, int64_t max_deg, int64_t* counts, void* stream);
+int spgnn_lstm_order_scatter(const int32_t* in_ptr, int64_t N, int64_t max_deg, const int64_t* offs,
+                             int32_t* perm, int32_t* rank, void* stream);
+int spgnn_lstm_cell_fwd(int64_t t, int64_t n_t, int64_t n_next, const int32_t* perm, const int32_t* in_ptr,
+                        const int32_t* in_src, const float* P, int64_t ldp, const float* R, int64_t ldr,
+                        uint16_t* gates, int64_t ldg, int64_t psg, const float* c_prev, float* c_cur,
+                        uint16_t* h_next, int64_t ldh, int64_t psh, float* out, int64_t ldo, int64_t D, void* stream);
+int spgnn_lstm_cell_bwd(int64_t t, int64_t n_t, int64_t n_next, const int32_t* perm, const float* g_out,
+                        int64_t ldgo, const float* dh_rec, int64_t ldr, float* dc, uint16_t* gates, int64_t ldg,
+                        int64_t psg, const float* c_prev, const float* c_cur, int64_t D, void* stream);
+int spgnn_lstm_dp(const uint16_t* dgates, int64_t ldg, int64_t psg, const int64_t* off, const int32_t* rank,
+                  const int32_t* in_ptr, const int32_t* out_ptr, const int32_t* out_dst, const int32_t* out_slot,
+                  float* dP, int64_t lddp, int64_t n_src, int64_t D, void* stream);
 
 /* Elementwise helpers the layer stacks need between projections.
  *   bias_act      : y = act(x + bias)           (GraphConv aggregate-first epilogue, GIN MLP, SAGE output)

@@ -1,5 +1,5 @@
 // Non-attention aggregations and the elementwise glue between projections:
-//   spmm            weighted neighbour sum with degree norms  (GraphConv 'both', GINConv 'mean')
+//   spmm            weighted neighbour sum with degree norms  (GraphConv 'both', GINConv 'mean', SAGEConv 'mean'/'gcn')
 //   sage_maxpool    elementwise neighbour max with arg-slot    (SAGEConv 'pool')
 //   bias_act / act_bwd / concat_dropout(+bwd)
 // One warp per node, lanes over 128-bit column chunks (scalar lanes when the width is not a multiple of 4).
@@ -52,7 +52,8 @@ __global__ void __launch_bounds__(kThreads) spmm_kernel(const float* __restrict_
                                                         const int32_t* __restrict__ ptr,
                                                         const int32_t* __restrict__ nbr,
                                                         const float* __restrict__ pre, const float* __restrict__ post,
-                                                        const float* __restrict__ self_eps,
+                                                        const float* __restrict__ self_eps, int self_in,
+                                                        int64_t n_self, const float* __restrict__ add, int64_t ld_add,
                                                         const float* __restrict__ bias, int act, float slope,
                                                         float* __restrict__ out, int64_t ldo, int64_t N, int F) {
     using V = Vec<VEC>;
@@ -63,6 +64,8 @@ __global__ void __launch_bounds__(kThreads) spmm_kernel(const float* __restrict_
     for (int64_t v = warp0; v < N; v += nwarps) {
         const int beg = __ldg(ptr + v), end = __ldg(ptr + v + 1);
         const float pv = post ? __ldg(post + v) : 1.f;
+        const bool has_self = v < n_self;
+        const float self_w = (self_in && has_self) ? (pre ? __ldg(pre + v) : 1.f) : 0.f;
         for (int col = lane * VEC; col < F; col += 32 * VEC) {
             typename V::T acc = V::zero();
             for (int s = beg; s < end; ++s) {
@@ -70,9 +73,11 @@ __global__ void __launch_bounds__(kThreads) spmm_kernel(const float* __restrict_
                 const float w = pre ? __ldg(pre + u) : 1.f;
                 acc = V::fma(w, V::ld(x + (int64_t)u * ldx + col), acc);
             }
-            // post-scale, self term, bias, activation
+            // self term inside the norm, post-scale, self term outside it, addend, bias, activation
+            if (self_w != 0.f) acc = V::fma(self_w, V::ld(x + v * ldx + col), acc);
             typename V::T r = V::fma(pv, acc, V::zero());
-            if (self_eps) r = V::fma(self_coef, V::ld(x + v * ldx + col), r);
+            if (self_eps && has_self) r = V::fma(self_coef, V::ld(x + v * ldx + col), r);
+            if (add) r = V::fma(1.f, V::ld(add + v * ld_add + col), r);
             if (bias) r = V::fma(1.f, V::ld(bias + col), r);
             r = V::map(r, [&](float t) { return act_fwd(t, act, slope); });
             V::st(out + v * ldo + col, r);
@@ -88,6 +93,11 @@ __global__ void degree_norms_kernel(const int32_t* __restrict__ ptr, int64_t N, 
         if (nsqrt) nsqrt[i] = powf(d, -0.5f);
         if (ninv) ninv[i] = 1.f / d;
     }
+}
+
+__global__ void inv_degree_kernel(const int32_t* __restrict__ ptr, int64_t N, float add, float* __restrict__ out) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x)
+        out[i] = 1.f / fmaxf((float)(ptr[i + 1] - ptr[i]) + add, 1.f);
 }
 
 template <int VEC>
@@ -263,16 +273,19 @@ static inline bool vec_ok(const void* p, int64_t ld, int64_t F) { return ((uintp
 using namespace spgnn;
 
 extern "C" int spgnn_spmm(const float* x, int64_t ldx, const int32_t* ptr, const int32_t* nbr, const float* pre,
-                          const float* post, const float* self_eps_ptr, const float* bias, int act, float slope,
-                          float* out, int64_t ldo, int64_t N, int64_t F, void* stream) {
-    SPGNN_REQUIRE(x && ptr && nbr && out && N > 0 && F > 0 && ldx >= F && ldo >= F, "spmm: bad argument");
+                          const float* post, const float* self_eps_ptr, int self_in, int64_t n_self, const float* add,
+                          int64_t ld_add, const float* bias, int act, float slope, float* out, int64_t ldo, int64_t N,
+                          int64_t F, void* stream) {
+    SPGNN_REQUIRE(x && ptr && nbr && out && N > 0 && F > 0 && ldx >= F && ldo >= F && n_self >= 0 && n_self <= N &&
+                  (!add || ld_add >= F), "spmm: bad argument");
     cudaStream_t st = as_stream(stream);
-    if (vec_ok(x, ldx, F) && vec_ok(out, ldo, F) && (!bias || ((uintptr_t)bias & 15) == 0))
-        spmm_kernel<4><<<node_grid(N), kThreads, 0, st>>>(x, ldx, ptr, nbr, pre, post, self_eps_ptr, bias, act, slope,
-                                                          out, ldo, N, (int)F);
+    if (vec_ok(x, ldx, F) && vec_ok(out, ldo, F) && (!bias || ((uintptr_t)bias & 15) == 0) &&
+        (!add || vec_ok(add, ld_add, F)))
+        spmm_kernel<4><<<node_grid(N), kThreads, 0, st>>>(x, ldx, ptr, nbr, pre, post, self_eps_ptr, self_in, n_self,
+                                                          add, ld_add, bias, act, slope, out, ldo, N, (int)F);
     else
-        spmm_kernel<1><<<node_grid(N), kThreads, 0, st>>>(x, ldx, ptr, nbr, pre, post, self_eps_ptr, bias, act, slope,
-                                                          out, ldo, N, (int)F);
+        spmm_kernel<1><<<node_grid(N), kThreads, 0, st>>>(x, ldx, ptr, nbr, pre, post, self_eps_ptr, self_in, n_self,
+                                                          add, ld_add, bias, act, slope, out, ldo, N, (int)F);
     SPGNN_LAUNCH_OK();
     return SPGNN_OK;
 }
@@ -280,6 +293,13 @@ extern "C" int spgnn_spmm(const float* x, int64_t ldx, const int32_t* ptr, const
 extern "C" int spgnn_degree_norms(const int32_t* ptr, int64_t N, float* norm_sqrt, float* norm_inv, void* stream) {
     SPGNN_REQUIRE(ptr && N > 0, "degree_norms: bad argument");
     degree_norms_kernel<<<elem_grid(N), kThreads, 0, as_stream(stream)>>>(ptr, N, norm_sqrt, norm_inv);
+    SPGNN_LAUNCH_OK();
+    return SPGNN_OK;
+}
+
+extern "C" int spgnn_inv_degree(const int32_t* ptr, int64_t N, float add, float* out, void* stream) {
+    SPGNN_REQUIRE(ptr && out && N > 0, "inv_degree: bad argument");
+    inv_degree_kernel<<<elem_grid(N), kThreads, 0, as_stream(stream)>>>(ptr, N, add, out);
     SPGNN_LAUNCH_OK();
     return SPGNN_OK;
 }

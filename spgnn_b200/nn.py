@@ -153,20 +153,50 @@ class GraphConv(nn.Module):
         return ops.linear(x, wt, self.bias, self._activation)
 
 
+class _LSTMParams(nn.Module):
+    """The parameters of ``nn.LSTM(D, D, batch_first=True)`` under its state-dict names, with its
+    ``reset_parameters``; the LSTM itself runs in ``ops.LstmReduceFn``."""
+
+    def __init__(self, D):
+        super().__init__()
+        self.hidden_size = D
+        self.weight_ih_l0 = nn.Parameter(torch.empty(4 * D, D))
+        self.weight_hh_l0 = nn.Parameter(torch.empty(4 * D, D))
+        self.bias_ih_l0 = nn.Parameter(torch.empty(4 * D))
+        self.bias_hh_l0 = nn.Parameter(torch.empty(4 * D))
+        self.reset_parameters()
+
+    def reset_parameters(self):
+        stdv = 1.0 / self.hidden_size ** 0.5
+        for w in self.parameters():
+            nn.init.uniform_(w, -stdv, stdv)
+
+
 class SAGEConv(nn.Module):
-    """``SAGEConv(in, out, aggregator_type='pool', feat_drop, activation, norm)`` (models.py:668-679)."""
+    """``SAGEConv(in, out, aggregator_type, feat_drop, activation, norm)`` (models.py:668-679) with DGL 0.7's four
+    aggregators: 'pool', 'mean', 'gcn' and 'lstm' (DESIGN.md §2).  Parameters and ``reset_parameters`` are DGL's:
+    'pool' has ``fc_pool``, 'lstm' has ``lstm`` (an ``nn.LSTM(in, in)``'s tensors), 'gcn' has no ``fc_self``."""
+
+    AGGREGATORS = ("pool", "mean", "gcn", "lstm")
 
     def __init__(self, in_feats, out_feats, aggregator_type="pool", feat_drop=0.0, bias=True, norm=None,
                  activation=None):
         super().__init__()
-        if aggregator_type != "pool":
-            raise SpgnnError("SAGEConv: only aggregator_type='pool' (the reference's setting) is implemented")
+        if aggregator_type not in self.AGGREGATORS:
+            raise SpgnnError(f"SAGEConv: aggregator_type must be one of {self.AGGREGATORS}, got {aggregator_type!r}")
+        self._aggre_type = aggregator_type
         self._in_feats, self._out_feats = in_feats, out_feats
         self.feat_drop_p = float(feat_drop)
         self.norm, self.activation = norm, activation
-        self.fc_pool = nn.Linear(in_feats, in_feats)
         per_linear = DGL_COMPAT["sage_bias_layout"] == "per_linear"
-        self.fc_self = nn.Linear(in_feats, out_feats, bias=per_linear)
+        if aggregator_type == "pool":
+            self.fc_pool = nn.Linear(in_feats, in_feats)
+        if aggregator_type == "lstm":
+            self.lstm = _LSTMParams(in_feats)
+        if aggregator_type != "gcn":
+            self.fc_self = nn.Linear(in_feats, out_feats, bias=per_linear)
+        else:
+            self.fc_self = None
         self.fc_neigh = nn.Linear(in_feats, out_feats, bias=per_linear)
         if not per_linear and bias:
             self.bias = nn.Parameter(torch.zeros(out_feats))
@@ -176,9 +206,19 @@ class SAGEConv(nn.Module):
 
     def reset_parameters(self):
         gain = nn.init.calculate_gain("relu")
-        nn.init.xavier_uniform_(self.fc_pool.weight, gain=gain)
-        nn.init.xavier_uniform_(self.fc_self.weight, gain=gain)
+        if self._aggre_type == "pool":
+            nn.init.xavier_uniform_(self.fc_pool.weight, gain=gain)
+        if self._aggre_type == "lstm":
+            self.lstm.reset_parameters()
+        if self._aggre_type != "gcn":
+            nn.init.xavier_uniform_(self.fc_self.weight, gain=gain)
         nn.init.xavier_uniform_(self.fc_neigh.weight, gain=gain)
+
+    def _bias(self):
+        b = self.bias
+        if b is None and self.fc_neigh.bias is not None:
+            b = self.fc_neigh.bias + (self.fc_self.bias if self.fc_self is not None else 0)
+        return b
 
     def forward(self, g, feat):
         """``g``: a batched Graph, or a sampled ``sampling.Block`` (``feat`` then has one row per SOURCE node and the
@@ -187,16 +227,36 @@ class SAGEConv(nn.Module):
         if is_block and feat.shape[0] != g.num_src_nodes:
             raise SpgnnError(f"SAGEConv: block has {g.num_src_nodes} source nodes, features have {feat.shape[0]} rows")
         h = ops.concat_dropout(feat, None, self.feat_drop_p, self.training)
-        m = ops.linear(h, self.fc_pool.weight, self.fc_pool.bias, "relu")
-        neigh = ops.MaxPoolFn.apply(m, g)
-        if is_block:
-            h = h[:g.num_dst_nodes]
-        # fc_self(h) + fc_neigh(neigh) as ONE two-source projection
-        w = torch.cat([self.fc_self.weight, self.fc_neigh.weight], 1)
-        b = self.bias
-        if b is None and self.fc_self.bias is not None:
-            b = self.fc_self.bias + self.fc_neigh.bias
-        rst = ops.linear(h, w, b, self.activation, x2=neigh)
+        h_dst = h[:g.num_dst_nodes] if is_block else h
+        b = self._bias()
+        lin_before_mp = self._in_feats > self._out_feats
+        agg = self._aggre_type
+        if agg == "mean" and lin_before_mp:
+            # mean_{u→v} fc_neigh(h)[u] + fc_self(h_dst) + bias, activation: self block and bias in the epilogue
+            x = ops.linear(h, self.fc_neigh.weight)
+            rst = ops.SpmmFn.apply(x, None, b, g, None, ops.inv_degree(g, 0), ops.act_code(self.activation), 0.0,
+                                   ops.linear(h_dst, self.fc_self.weight))
+        elif agg == "gcn":
+            # (Σ_{u→v} x[u] + x[v]) / (in_deg(v) + 1), x = fc_neigh(h) before or after the aggregation
+            if lin_before_mp:
+                rst = ops.SpmmFn.apply(ops.linear(h, self.fc_neigh.weight), None, b, g, None, ops.inv_degree(g, 1),
+                                       ops.act_code(self.activation), 0.0, None, True)
+            else:
+                neigh = ops.SpmmFn.apply(h, None, None, g, None, ops.inv_degree(g, 1), 0, 0.0, None, True)
+                rst = ops.linear(neigh, self.fc_neigh.weight, b, self.activation)
+        else:
+            if agg == "pool":
+                m = ops.linear(h, self.fc_pool.weight, self.fc_pool.bias, "relu")
+                neigh = ops.MaxPoolFn.apply(m, g)
+            elif agg == "mean":
+                neigh = ops.SpmmFn.apply(h, None, None, g, None, ops.inv_degree(g, 0), 0, 0.0)
+            else:
+                lp = self.lstm
+                P = ops.linear(h, lp.weight_ih_l0, lp.bias_ih_l0 + lp.bias_hh_l0)
+                neigh = ops.LstmReduceFn.apply(P, lp.weight_hh_l0, g)
+            # fc_self(h_dst) + fc_neigh(neigh) as ONE two-source projection
+            w = torch.cat([self.fc_self.weight, self.fc_neigh.weight], 1)
+            rst = ops.linear(h_dst, w, b, self.activation, x2=neigh)
         return self.norm(rst) if self.norm is not None else rst
 
 

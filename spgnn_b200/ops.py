@@ -479,27 +479,33 @@ class GatAggFn(Function):
 
 
 class SpmmFn(Function):
-    """out = act(post ⊙ Σ_{u→v} pre[u]·x[u] + (1+eps)·x[v]·[eps given] + bias)  — GraphConv / GINConv-mean."""
+    """out = act(post ⊙ (Σ_{u→v} pre[u]·x[u] + [self_in] pre[v]·x[v]) + (1+eps)·x[v]·[eps given] + add[v] + bias)
+    — GraphConv / GINConv-mean / SAGEConv mean and gcn.  ``graph`` is a batched Graph (output rows = nodes) or a
+    sampled ``sampling.Block`` (rows of ``x`` = source nodes, output rows = destination nodes; the self terms read
+    x[v] for the destinations, which are the first source rows)."""
 
     @staticmethod
-    def forward(ctx, x, eps, bias, graph, pre, post, act, slope):
-        require_cuda(x, eps, bias)
+    def forward(ctx, x, eps, bias, graph, pre, post, act, slope, add=None, self_in=False):
+        require_cuda(x, eps, bias, add)
         x = _rows(x)
-        N, F = x.shape
+        n_src, F = x.shape
+        N = _n_dst(graph)
         out = empty_padded(N, F, x.device)
         b = bias.contiguous() if bias is not None else None
-        lib().spmm(ptr(x), x.stride(0), ptr(graph.in_ptr), ptr(graph.in_src), ptr(pre), ptr(post), ptr(eps), ptr(b),
-                   act, float(slope), ptr(out), out.stride(0), N, F, stream(),
-                   _key=("bytes", 8.0 * N * F + 4.0 * (N + 1) + 4.0 * graph.num_edges))
+        a = _rows(add) if add is not None else None
+        lib().spmm(ptr(x), x.stride(0), ptr(graph.in_ptr), ptr(graph.in_src), ptr(pre), ptr(post), ptr(eps),
+                   int(self_in), N, ptr(a), a.stride(0) if a is not None else 0, ptr(b), act, float(slope), ptr(out),
+                   out.stride(0), N, F, stream(),
+                   _key=("bytes", 4.0 * (n_src + N * (2 if a is not None else 1)) * F + 4.0 * (N + 1) + 4.0 * graph.num_edges))
         ctx.save_for_backward(x if eps is not None else None, eps, out if act else None)
         ctx.graph, ctx.pre, ctx.post = graph, pre, post
-        ctx.cfg = (act, float(slope), b is not None)
+        ctx.cfg = (act, float(slope), b is not None, bool(self_in), n_src)
         return out
 
     @staticmethod
     def backward(ctx, g):
         x, eps, out = ctx.saved_tensors
-        act, slope, has_bias = ctx.cfg
+        act, slope, has_bias, self_in, n_src = ctx.cfg
         gr = ctx.graph
         L = lib()
         g = _rows(g)
@@ -510,16 +516,160 @@ class SpmmFn(Function):
             g = d
         dx = deps = db = None
         if ctx.needs_input_grad[0]:
-            dx = empty_padded(N, F, g.device)
-            # transpose graph: out-edges, with the roles of the two norms swapped
-            L.spmm(ptr(g), g.stride(0), ptr(gr.out_ptr), ptr(gr.out_dst), ptr(ctx.post), ptr(ctx.pre), ptr(eps), None,
-                   0, 0.0, ptr(dx), dx.stride(0), N, F, stream(),
-                   _key=("bytes", 8.0 * N * F + 4.0 * (N + 1) + 4.0 * gr.num_edges))
+            dx = empty_padded(n_src, F, g.device)
+            # transpose graph: out-edges into the source rows, with the roles of the two norms swapped; the self terms
+            # exist for the first N (destination) rows only
+            L.spmm(ptr(g), g.stride(0), ptr(gr.out_ptr), ptr(gr.out_dst), ptr(ctx.post), ptr(ctx.pre), ptr(eps),
+                   int(self_in), N, None, 0, None, 0, 0.0, ptr(dx), dx.stride(0), n_src, F, stream(),
+                   _key=("bytes", 4.0 * (n_src + N) * F + 4.0 * (n_src + 1) + 4.0 * gr.num_edges))
         if eps is not None and ctx.needs_input_grad[1]:
-            deps = (g * x).sum().reshape(1)
+            deps = (g * x[:N]).sum().reshape(1)
         if has_bias and ctx.needs_input_grad[2]:
             db = colsum(g)
-        return dx, deps, db, None, None, None, None, None
+        need = ctx.needs_input_grad
+        dadd = g if len(need) > 8 and need[8] else None
+        return (dx, deps, db, None, None, None, None, None, dadd, None)[:len(need)]
+
+
+def _n_dst(graph):
+    return int(graph.num_dst_nodes) if getattr(graph, "is_block", False) else int(graph.num_nodes)
+
+
+def inv_degree(graph, add):
+    """1 / max(in_degree + add, 1) per destination node (SAGEConv mean: add 0, gcn: add 1), cached on the graph."""
+    cache = graph.__dict__.setdefault("_inv_degree", {})
+    hit = cache.get(add)
+    if hit is None:
+        n = _n_dst(graph)
+        hit = torch.empty(n, dtype=torch.float32, device=graph.in_ptr.device)
+        lib().inv_degree(ptr(graph.in_ptr), n, float(add), ptr(hit), stream())
+        cache[add] = hit
+    return hit
+
+
+class LstmOrder:
+    """Destinations sorted by in-degree, descending and stable (a device counting sort): ``perm[row]`` = destination,
+    ``rank[destination]`` = row; ``steps[t]`` = n_t = destinations with in-degree > t, so LSTM step t runs over rows
+    [0, n_t); ``off[t]`` = Σ_{s<t} n_s is where step t's rows start in the per-step buffers (int64, host and device).
+    Built once per graph (two small device→host reads) and cached on it, like ``Graph.norms()``."""
+
+    def __init__(self, graph):
+        L = lib()
+        dev = graph.in_ptr.device
+        n = _n_dst(graph)
+        self.n = n
+        deg = graph.in_ptr[1:n + 1] - graph.in_ptr[:n]
+        max_deg = int(deg.max().item()) if n > 0 else 0
+        chunks = (n + 255) // 256
+        counts = torch.empty((max_deg + 1) * chunks, dtype=torch.int64, device=dev)
+        L.lstm_order_count(ptr(graph.in_ptr), n, max_deg, ptr(counts), stream())
+        from .graph import device_scan
+        offs = device_scan(counts)
+        self.perm = torch.empty(n, dtype=torch.int32, device=dev)
+        self.rank = torch.empty(n, dtype=torch.int32, device=dev)
+        L.lstm_order_scatter(ptr(graph.in_ptr), n, max_deg, ptr(offs), ptr(self.perm), ptr(self.rank), stream())
+        # bucket of degree d starts at offs[(max_deg - d) * chunks]: the rows before it have degree > d
+        self.steps = offs[torch.arange(max_deg, 0, -1, device=dev) * chunks].tolist()     # d = 0 .. max_deg - 1
+        self.off = [0]
+        for k in self.steps:
+            self.off.append(self.off[-1] + k)
+        self.off_dev = torch.tensor(self.off, dtype=torch.int64, device=dev)
+
+
+def lstm_order(graph):
+    o = graph.__dict__.get("_lstm_order")
+    if o is None:
+        o = graph.__dict__["_lstm_order"] = LstmOrder(graph)
+    return o
+
+
+class LstmReduceFn(Function):
+    """neigh[v] = h_T(v) of DGL 0.7's ``_lstm_reducer``: an LSTM (zero initial state, gates i, f, g, o) over the
+    messages of v's in-edges in in-CSC order.  ``P`` = X·W_ihᵀ + b_ih + b_hh [n_src, 4D] is the input projection
+    (``linear``: autograd takes its gradients), ``W_hh`` [4D, D].  Returns [n_dst, D]; zero for in-degree 0.
+
+    Step t runs over the first n_t rows of ``LstmOrder`` (destinations by descending in-degree); step 0 needs no
+    GEMM (h_0 = 0), step t ≥ 1 adds R_t = H_{t-1}[:n_t]·W_hhᵀ from the planes GEMMs whatever ``GEMM_MODE`` says.
+    Per-step buffers hold step t at rows [off_t, off_t + n_t): the gate activations (as the 16-bit halves of the
+    planes the backward overwrites with the gate gradients), c, and h as planes at the rows of the step that reads
+    it, so dW_hh is ONE GEMM over all steps."""
+
+    @staticmethod
+    def forward(ctx, P, W_hh, graph):
+        from . import stack
+        require_cuda(P, W_hh)
+        P, W = _rows(P), _rows(W_hh)
+        D = W.shape[1]
+        if W.shape[0] != 4 * D or P.shape[1] != 4 * D:
+            raise SpgnnError(f"lstm reducer: W_hh {tuple(W.shape)} and P {tuple(P.shape)} do not match an LSTM")
+        if D % 4:
+            raise SpgnnError(f"lstm reducer: the feature width must be a multiple of 4, got {D}")
+        if P.stride(0) % 4 or P.data_ptr() % 16:
+            P = empty_padded(P.shape[0], 4 * D, P.device).copy_(P)
+        o = lstm_order(graph)
+        dev = P.device
+        out = torch.zeros(o.n, _pad4(D), dtype=torch.float32, device=dev)[:, :D]
+        ctx.graph, ctx.order, ctx.n_src, ctx.rec = graph, o, P.shape[0], None
+        ctx.save_for_backward(W)
+        T = len(o.steps)
+        if T == 0:
+            return out
+        E, n0 = o.off[-1], o.steps[0]
+        G = stack.Planes(E, 4 * D, dev)
+        C = torch.empty(E, D, dtype=torch.float32, device=dev)
+        Hn = stack.Planes(E - n0, D, dev) if T > 1 else None
+        R = torch.empty(o.steps[1], 4 * D, dtype=torch.float32, device=dev) if T > 1 else None
+        L = lib()
+        for t in range(T):
+            n_t, n_next = o.steps[t], (o.steps[t + 1] if t + 1 < T else 0)
+            Rt = None
+            if t > 0:
+                Rt = stack.planes_linear(stack.PlanesView(Hn, 0, D, o.off[t] - n0, n_t), W, out=R[:n_t])
+            hn = Hn.ptr() + 2 * (o.off[t + 1] - n0) * Hn.ld if n_next else None
+            L.lstm_cell_fwd(t, n_t, n_next, ptr(o.perm), ptr(graph.in_ptr), ptr(graph.in_src), ptr(P), P.stride(0),
+                            ptr(Rt), R.stride(0) if Rt is not None else 0, G.ptr() + 2 * o.off[t] * G.ld, G.ld, G.ps,
+                            ptr(C[o.off[t - 1]:]) if t > 0 else None, ptr(C[o.off[t]:]), hn,
+                            Hn.ld if Hn is not None else 0, Hn.ps if Hn is not None else 0, ptr(out), out.stride(0), D,
+                            stream(), _name="lstm_cell_fwd",
+                            _key=("bytes", n_t * (40.0 * D + (20.0 * D if t > 0 else 0.0) + 12.0)))
+        ctx.rec = (G, C, Hn)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        from . import stack
+        (W,) = ctx.saved_tensors
+        o, graph, n_src = ctx.order, ctx.graph, ctx.n_src
+        D = W.shape[1]
+        dev = W.device
+        dP = empty_padded(n_src, 4 * D, dev)
+        T = len(o.steps)
+        if T == 0:
+            return dP.zero_(), torch.zeros_like(W), None
+        G, C, Hn = ctx.rec
+        ctx.rec = None
+        g = _rows(g)
+        if g.stride(0) % 4 or g.data_ptr() % 16:
+            g = empty_padded(g.shape[0], D, dev).copy_(g)
+        E, n0 = o.off[-1], o.steps[0]
+        dH = torch.empty(o.steps[1], D, dtype=torch.float32, device=dev) if T > 1 else None
+        dc = torch.empty(o.steps[1], D, dtype=torch.float32, device=dev) if T > 1 else None
+        L = lib()
+        for t in reversed(range(T)):
+            n_t, n_next = o.steps[t], (o.steps[t + 1] if t + 1 < T else 0)
+            L.lstm_cell_bwd(t, n_t, n_next, ptr(o.perm), ptr(g), g.stride(0), ptr(dH) if n_next else None, D,
+                            ptr(dc) if (t > 0 or n_next) else None, G.ptr() + 2 * o.off[t] * G.ld, G.ld, G.ps,
+                            ptr(C[o.off[t - 1]:]) if t > 0 else None, ptr(C[o.off[t]:]), D, stream(),
+                            _name="lstm_cell_bwd",
+                            _key=("bytes", n_t * (40.0 * D + (8.0 * D if t > 0 else 0.0) + (4.0 * D if n_next else 0.0))))
+            if t > 0:
+                stack.planes_linear_bwd_input(stack.PlanesView(G, 0, 4 * D, o.off[t], n_t), W, D, out=dH[:n_t])
+        dW = (stack.planes_linear_bwd_weight(stack.PlanesView(G, 0, 4 * D, n0, E - n0), Hn) if T > 1
+              else torch.zeros_like(W))
+        L.lstm_dp(G.ptr(), G.ld, G.ps, ptr(o.off_dev), ptr(o.rank), ptr(graph.in_ptr), ptr(graph.out_ptr),
+                  ptr(graph.out_dst), ptr(graph.out_slot), ptr(dP), dP.stride(0), n_src, D, stream(),
+                  _key=("bytes", 16.0 * D * (E + n_src) + 16.0 * E))
+        return dP, dW, None
 
 
 class MaxPoolFn(Function):

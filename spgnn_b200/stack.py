@@ -124,13 +124,14 @@ class Planes:
 
 
 class PlanesView:
-    """Columns [col0, col0 + cols) of a Planes (same rows, ld and plane stride)."""
+    """Columns [col0, col0 + cols) and rows [row0, row0 + rows) of a Planes (same ld and plane stride)."""
 
     __slots__ = ("buf", "rows", "cols", "ld", "ps", "_p")
 
-    def __init__(self, base, col0, cols):
-        self.buf, self.rows, self.cols, self.ld, self.ps = base.buf, base.rows, int(cols), base.ld, base.ps
-        self._p = base.ptr(int(col0))
+    def __init__(self, base, col0, cols, row0=0, rows=None):
+        self.buf, self.cols, self.ld, self.ps = base.buf, int(cols), base.ld, base.ps
+        self.rows = base.rows - int(row0) if rows is None else int(rows)
+        self._p = base.ptr(int(col0)) + 2 * int(row0) * base.ld
 
     def ptr(self, col=0):
         return self._p + 2 * col
@@ -155,8 +156,9 @@ def _ws(nbytes, device):
     return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
 
 
-def planes_linear(A1: Planes, W, bias=None, act=0, slope=0.0, A2: Planes | None = None):
-    """fp32 [M, N] = [A1 | A2] @ W^T (+bias)(act); W fp32 [N, K1+K2] with unit inner stride."""
+def planes_linear(A1: Planes, W, bias=None, act=0, slope=0.0, A2: Planes | None = None, out=None):
+    """fp32 [M, N] = [A1 | A2] @ W^T (+bias)(act); W fp32 [N, K1+K2] with unit inner stride.  ``out``: an [M, N]
+    destination with 16-byte aligned rows (a buffer reused across calls)."""
     W = ops._rows(W)
     M, N = A1.rows, W.shape[0]
     K1, K2 = A1.cols, (A2.cols if A2 is not None else 0)
@@ -164,8 +166,11 @@ def planes_linear(A1: Planes, W, bias=None, act=0, slope=0.0, A2: Planes | None 
         raise SpgnnError(f"planes_linear: weight has {W.shape[1]} columns, input has {K1}+{K2}")
     # rows padded to 128 bytes once they are wide enough to be sliced by the per-tree layer kernels (TMA boxes of 32
     # columns then start on cache-line boundaries)
-    C = ops.empty_padded(M, N, W.device) if N < 64 else torch.empty(
-        M, (N + 31) // 32 * 32, dtype=torch.float32, device=W.device)[:, :N]
+    if out is not None:
+        C = out
+    else:
+        C = ops.empty_padded(M, N, W.device) if N < 64 else torch.empty(
+            M, (N + 31) // 32 * 32, dtype=torch.float32, device=W.device)[:, :N]
     L = lib()
     ws = _ws(L.planes_linear_fwd_ws(N, K1, K2), W.device)
     L.planes_linear_fwd(A1.ptr(), A1.ld, A1.ps, K1, A2.ptr() if A2 is not None else None,
