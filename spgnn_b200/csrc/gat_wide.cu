@@ -501,6 +501,20 @@ extern "C" int spgnn_gat_aggx_fwd(const spgnn_gat_wide* L, void* stream) {
     return SPGNN_OK;
 }
 
+// the most dynamic shared memory one block can opt into on sm_100
+constexpr size_t kBwdSmemMax = 227 * 1024;
+#define WIDE_INSTANCES(KERNEL)                                                                                 \
+    (const void*)KERNEL<1, 16>, (const void*)KERNEL<1, 32>, (const void*)KERNEL<2, 16>, (const void*)KERNEL<2, 32>, \
+        (const void*)KERNEL<4, 16>, (const void*)KERNEL<4, 32>
+static cudaError_t set_bwd_smem() {
+    const void* fns[] = {WIDE_INSTANCES(aggx_bwd_dst_kernel), WIDE_INSTANCES(aggx_bwd_src_kernel)};
+    for (const void* f : fns) {
+        const cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmemMax);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 extern "C" int spgnn_gat_aggx_bwd(const spgnn_gat_wide* L, void* stream) {
     WArgs a{};
     int rc = fill(a, L, true);
@@ -508,7 +522,14 @@ extern "C" int spgnn_gat_aggx_bwd(const spgnn_gat_wide* L, void* stream) {
     cudaStream_t st = as_stream(stream);
     const unsigned grid = wide_grid(a.N);
     const size_t smem = stage_bytes(a.H, a.k4);
-    SPGNN_REQUIRE(smem <= 48 * 1024, "gat_aggx_bwd: k_in too large for the logit-weight stage (%zu bytes)", smem);
+    // The logit-weight stage grows with k_in: past 48 KB (H = 4 above k_in = 415) the kernels opt into more dynamic
+    // shared memory, so every layer StackPlan marks wide (H*F <= 8192, k_in <= H*F / 4: at most 101 KB) trains.
+    SPGNN_REQUIRE(smem <= kBwdSmemMax, "gat_aggx_bwd: k_in too large for the logit-weight stage (%zu bytes)", smem);
+    static DeviceOnce attr;
+    if (smem > 48 * 1024 && attr.pending()) {
+        SPGNN_CUDA_OK(set_bwd_smem());
+        attr.done();
+    }
     WIDE_DISPATCH(aggx_bwd_dst_kernel, a.k4 >> 2, a);
     WIDE_DISPATCH(aggx_bwd_src_kernel, a.k4 >> 2, a);
     return SPGNN_OK;

@@ -222,6 +222,14 @@ extern "C" int spgnn_lstm_order_scatter(const int32_t* in_ptr, int64_t N, int64_
                                         int32_t* perm, int32_t* rank, void* stream) {
     SPGNN_REQUIRE(in_ptr && offs && perm && rank && N > 0 && max_deg >= 0, "lstm_order_scatter: bad argument");
     SPGNN_REQUIRE(max_deg < kMaxSortKeys, "lstm_order_scatter: in-degree above the sort's key range");
+    // max_deg + 2 keys (the padding lanes of the last chunk take key max_deg + 1): at max_deg = kMaxSortKeys - 1 that
+    // is 4 bytes over the 48 KB a launch gets without opting in
+    static DeviceOnce attr;
+    if (attr.pending()) {
+        SPGNN_CUDA_OK(cudaFuncSetAttribute(order_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)((kMaxSortKeys + 1) * sizeof(int))));
+        attr.done();
+    }
     const unsigned chunks = (unsigned)ceil_div(N, kSortChunk);
     order_scatter_kernel<<<chunks, kSortChunk, (size_t)(max_deg + 2) * sizeof(int), as_stream(stream)>>>(
         in_ptr, N, max_deg, offs, perm, rank);
