@@ -38,7 +38,7 @@ extern "C" {
 #define SPGNN_ACT_ELU  1
 #define SPGNN_ACT_TANH 2
 #define SPGNN_ACT_RELU 3
-#define SPGNN_ACT_LEAKY 4      /* slope passed separately */
+#define SPGNN_ACT_LEAKY 4      /* slope passed separately; the GAT layer entry points use F.leaky_relu's 0.01 */
 
 const char* spgnn_last_error(void);
 int  spgnn_abi_version(void);

@@ -84,10 +84,15 @@ __device__ __forceinline__ float exp_fast(float x) {
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x * 1.4426950408889634f));
     return y;
 }
+// Slope of SPGNN_ACT_LEAKY as the activation of a GAT layer (gat.cu, gat_layer.cu, gat_tree.cu and the aggregate-first
+// output layer of gemm_tma.cu): GATConv takes its activation as a callable, and F.leaky_relu applies its default
+// negative_slope of 0.01.  Kernels whose activation comes with an explicit slope (linear, spmm, max-pool) pass it.
+constexpr float kGatLeakySlope = 0.01f;
 __device__ __forceinline__ float act_fast(float x, int act) {
     if (act == SPGNN_ACT_ELU) return x > 0.f ? x : exp_fast(x) - 1.f;
     if (act == SPGNN_ACT_TANH) return 1.f - __fdividef(2.f, exp_fast(2.f * x) + 1.f);
     if (act == SPGNN_ACT_RELU) return fmaxf(x, 0.f);
+    if (act == SPGNN_ACT_LEAKY) return x > 0.f ? x : kGatLeakySlope * x;
     return x;
 }
 // derivative expressed through the OUTPUT y = act(x)

@@ -320,7 +320,7 @@ __device__ __forceinline__ float act_slope(float x, int act) {
         const float y = 1.f - __fdividef(2.f, exp_fast(2.f * x) + 1.f);
         return 1.f - y * y;
     }
-    return act_grad_from_out(act_fast(x, act), act, 0.f);
+    return act_grad_from_out(act_fast(x, act), act, kGatLeakySlope);
 }
 template <int ACT>
 __device__ __forceinline__ float4 act_slope4(float4 p, int act) {

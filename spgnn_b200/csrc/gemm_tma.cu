@@ -459,20 +459,20 @@ template <int ACT>
 __device__ __forceinline__ float wide_act(float x, int act) {
     if (ACT == SPGNN_ACT_ELU) return x > 0.f ? x : exp_fast(x) - 1.f;     // FMUL + MUFU.EX2 + FADD on the x <= 0 side
     if (ACT == SPGNN_ACT_NONE) return x;
-    return act_fwd(x, act, 0.f);
+    return act_fwd(x, act, kGatLeakySlope);
 }
 template <int ACT>
 __device__ __forceinline__ float wide_act_grad(float y, int act) {
     if (ACT == SPGNN_ACT_ELU) return y > 0.f ? 1.f : y + 1.f;
     if (ACT == SPGNN_ACT_NONE) return 1.f;
-    return act_grad_from_out(y, act, 0.f);
+    return act_grad_from_out(y, act, kGatLeakySlope);
 }
 // act(x) and act'(x) from the pre-activation in one go (ELU: one exponential serves both)
 template <int ACT>
 __device__ __forceinline__ float wide_act_grad_pre(float x, int act) {
     if (ACT == SPGNN_ACT_ELU) return x > 0.f ? 1.f : exp_fast(x);
     if (ACT == SPGNN_ACT_NONE) return 1.f;
-    return act_grad_from_out(act_fwd(x, act, 0.f), act, 0.f);
+    return act_grad_from_out(act_fwd(x, act, kGatLeakySlope), act, kGatLeakySlope);
 }
 __device__ __forceinline__ void st_planes4(__nv_bfloat16* q, int64_t ps, float4 d) {
     uint32_t h0, l0, h1, l1;

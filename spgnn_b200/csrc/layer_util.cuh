@@ -23,8 +23,8 @@ __device__ __forceinline__ float4 act4(float4 p, int act) {
     return make_float4(act_fast(p.x, act), act_fast(p.y, act), act_fast(p.z, act), act_fast(p.w, act));
 }
 __device__ __forceinline__ float4 actgrad4(float4 y, int act) {
-    return make_float4(act_grad_from_out(y.x, act, 0.f), act_grad_from_out(y.y, act, 0.f),
-                       act_grad_from_out(y.z, act, 0.f), act_grad_from_out(y.w, act, 0.f));
+    return make_float4(act_grad_from_out(y.x, act, kGatLeakySlope), act_grad_from_out(y.y, act, kGatLeakySlope),
+                       act_grad_from_out(y.z, act, kGatLeakySlope), act_grad_from_out(y.w, act, kGatLeakySlope));
 }
 __device__ __forceinline__ float leaky(float x, float slope) { return x > 0.f ? x : slope * x; }
 
