@@ -477,6 +477,21 @@ int spgnn_seed_salt_units(void);
  *   g = nesterov ? g + mu*buf : buf;  p -= lr*g.   buf may be null when mu == 0. */
 int spgnn_sgd_step(float* p, const float* g, float* buf, int64_t n, float lr, float mu, float dampening,
                    float weight_decay, int nesterov, float grad_scale, int first_step, void* stream);
+/* torch.optim.Adam (decoupled = 0) / AdamW (decoupled = 1) over the live chunks of a flat bucket, as torch's
+ * _single_tensor_adam.  chunks: int64 [n_chunks, 3] = {offset, length, parameter index}, each chunk inside one
+ * parameter and inside the buckets (not checked); live: int64 [n_live], the distinct indices of the parameters that
+ * have a gradient this step.  steps: int64 per parameter, in device memory: the call first adds 1 to steps[live[i]]
+ * (its own launch), then for every element of every chunk, with t = steps[parameter]:
+ *   g = maximize ? -g : g;  Adam: g += weight_decay*p   AdamW: p *= 1 - lr*weight_decay   (weight_decay != 0);
+ *   m = lerp(m, g, 1-beta1);  v = beta2*v + (1-beta2)*g^2;  amsgrad: vmax = max(vmax, v), used in place of v;
+ *   p -= (lr / (1 - beta1^t)) * m / (sqrt(v) / sqrt(1 - beta2^t) + eps)   (bias corrections in fp64).
+ * t never comes from the host, so a CUDA graph that captured this call advances it on every replay.  Elements
+ * outside the chunks are not touched.  betas in [0, 1), lr, eps, weight_decay >= 0; max_exp_avg_sq non-null iff
+ * amsgrad; p, g, exp_avg, exp_avg_sq, max_exp_avg_sq 16-byte aligned.  Two launches. */
+int spgnn_adam_step(float* p, const float* g, float* exp_avg, float* exp_avg_sq, float* max_exp_avg_sq,
+                    int64_t* steps, const int64_t* chunks, int64_t n_chunks, const int64_t* live, int64_t n_live,
+                    double lr, double beta1, double beta2, double eps, double weight_decay, int amsgrad, int maximize,
+                    int decoupled, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Wire format of a scan batch (host loader -> device batch builder; replaces the dense per-scan H2D copies of

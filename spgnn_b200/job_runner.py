@@ -196,13 +196,24 @@ class GCNTrain(_Runner):
         s = self.settings
         self.model.set_gcn_only()
         opt_kw = dict(s.OPTIMIZER)
-        if not opt_kw.pop("method", "torch.optim.SGD").endswith("SGD"):
-            raise SpgnnError("only torch.optim.SGD is implemented for the device optimiser")
-        unknown = set(opt_kw) - {"lr", "momentum", "dampening", "weight_decay", "nesterov"}
-        if unknown:          # e.g. 'groups', 'maximize', 'foreach': refuse rather than train differently in silence
-            raise SpgnnError(f"OPTIMIZER keys {sorted(unknown)} are not supported by the device optimiser")
-        opt_kw.setdefault("lr", 1e-4)
-        self.optimizer = runner.FlatSGD(self.model.parameters(), **opt_kw)
+        method = opt_kw.pop("method", "torch.optim.SGD")
+        name = method.rpartition(".")[2]
+        if name in ("Adam", "AdamW"):
+            unknown = set(opt_kw) - {"lr", "betas", "eps", "weight_decay", "amsgrad", "maximize"}
+            if unknown:      # e.g. 'foreach', 'fused', 'capturable': refuse rather than train differently in silence
+                raise SpgnnError(f"OPTIMIZER keys {sorted(unknown)} are not supported by the device optimiser")
+            opt_kw.setdefault("lr", 1e-3)                  # torch's defaults; AdamW decays by 0.01 unless told
+            if name == "AdamW":
+                opt_kw.setdefault("weight_decay", 1e-2)
+            self.optimizer = runner.FlatAdam(self.model.parameters(), decoupled=name == "AdamW", **opt_kw)
+        else:
+            if not method.endswith("SGD"):
+                raise SpgnnError("only torch.optim.SGD, Adam and AdamW are implemented for the device optimiser")
+            unknown = set(opt_kw) - {"lr", "momentum", "dampening", "weight_decay", "nesterov"}
+            if unknown:      # e.g. 'groups', 'maximize', 'foreach': refuse rather than train differently in silence
+                raise SpgnnError(f"OPTIMIZER keys {sorted(unknown)} are not supported by the device optimiser")
+            opt_kw.setdefault("lr", 1e-4)
+            self.optimizer = runner.FlatSGD(self.model.parameters(), **opt_kw)
         self.base_lr = self.optimizer.lr
         sched_kw = dict(s.SCHEDULER)
         if not sched_kw.pop("method", "torch.optim.lr_scheduler.ExponentialLR").endswith("ExponentialLR"):

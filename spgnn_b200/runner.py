@@ -1,5 +1,5 @@
 """Callers of the hot path, kept on device: batch assembly from host buffers, the training step of
-/root/reference/job_runner.py:1863-1920 (GCNTrainSPGNN.train) / :1368-1416 (GCNTrain.train) and the SGD update.
+/root/reference/job_runner.py:1863-1920 (GCNTrainSPGNN.train) / :1368-1416 (GCNTrain.train) and the SGD or Adam update.
 
 One process per GPU; trees shard by graph (they are independent components, SURVEY.md §8e): inference needs no
 collective, training adds ONE NCCL all-reduce of the flat gradient bucket per step, and the masked weighted
@@ -16,29 +16,21 @@ from ._lib import lib, ptr, stream
 CLASS_WEIGHTS_22 = [0.2] + [0.8] * 21      # exp_settings/st_pgat_spgnn_3.py:70-74 via job_runner.py:1867
 
 
-class FlatSGD:
-    """torch.optim.SGD semantics (momentum, dampening, weight_decay, nesterov; the reference builds
-    ``torch.optim.SGD(model.parameters(), **settings.OPTIMIZER)``, job_runner.py:239-249) over ONE flat fp32 bucket:
-    parameters are views into one contiguous buffer and a step is one multi-tensor gather of the gradients into a
-    second one, one all-reduce (when world_size > 1) and one fused update kernel.  ``zero_grad`` drops the gradients
-    (``p.grad = None``), so autograd hands over each parameter's gradient without an accumulation kernel per
-    parameter — at the reference's own batch size (64 trees) a step is launch-bound and those ~40 tiny kernels are
-    a tenth of it.  As in torch, a parameter whose ``grad`` is None is skipped entirely (no momentum-only update, no
-    weight decay) and its momentum buffer starts at the first gradient it receives."""
+class _FlatBucket:
+    """The parameters as views into ONE contiguous fp32 buffer and a second one their gradients are gathered into:
+    a step is one multi-tensor gather, one all-reduce (when world_size > 1) and the optimiser's fused update over
+    the buffer.  ``zero_grad`` drops the gradients (``p.grad = None``), so autograd hands over each parameter's
+    gradient without an accumulation kernel per parameter — at the reference's own batch size (64 trees) a step is
+    launch-bound and those ~40 tiny kernels are a tenth of it."""
 
-    def __init__(self, params, lr, momentum=0.0, dampening=0.0, weight_decay=0.0, nesterov=False, process_group=None):
+    def __init__(self, params, process_group=None):
         self.params = [p for p in params if p.requires_grad]
-        self.lr, self.momentum = float(lr), float(momentum)
-        self.dampening, self.weight_decay, self.nesterov = float(dampening), float(weight_decay), bool(nesterov)
-        if self.nesterov and (self.momentum <= 0.0 or self.dampening != 0.0):
-            raise ValueError("Nesterov momentum requires a momentum and zero dampening")        # torch's own check
         self.group = process_group
         self.world = dist.get_world_size(process_group) if dist.is_available() and dist.is_initialized() else 1
         n = sum(p.numel() for p in self.params)
         dev = self.params[0].device
         self.flat_p = torch.empty(n, dtype=torch.float32, device=dev)
         self.flat_g = torch.zeros(n, dtype=torch.float32, device=dev)
-        self.buf = torch.zeros(n, dtype=torch.float32, device=dev)
         self.g_views, self.offsets = [], []
         o = 0
         for p in self.params:
@@ -49,7 +41,6 @@ class FlatSGD:
             self.offsets.append((o, k))
             p.grad = None
             o += k
-        self.has_buf = [False] * len(self.params)       # momentum buffer initialised (torch: state['momentum_buffer'])
         self.steps = 0
         self.numel = n
 
@@ -82,6 +73,26 @@ class FlatSGD:
             self.params[i].grad = self.g_views[i]
         return live
 
+    def set_lr(self, lr):
+        self.lr = float(lr)
+
+
+class FlatSGD(_FlatBucket):
+    """torch.optim.SGD semantics (momentum, dampening, weight_decay, nesterov; the reference builds
+    ``torch.optim.SGD(model.parameters(), **settings.OPTIMIZER)``, job_runner.py:239-249) over the flat bucket: one
+    fused update kernel per contiguous run of live parameters.  As in torch, a parameter whose ``grad`` is None is
+    skipped entirely (no momentum-only update, no weight decay) and its momentum buffer starts at the first gradient
+    it receives."""
+
+    def __init__(self, params, lr, momentum=0.0, dampening=0.0, weight_decay=0.0, nesterov=False, process_group=None):
+        self.lr, self.momentum = float(lr), float(momentum)
+        self.dampening, self.weight_decay, self.nesterov = float(dampening), float(weight_decay), bool(nesterov)
+        if self.nesterov and (self.momentum <= 0.0 or self.dampening != 0.0):
+            raise ValueError("Nesterov momentum requires a momentum and zero dampening")        # torch's own check
+        super().__init__(params, process_group)
+        self.buf = torch.zeros(self.numel, dtype=torch.float32, device=self.flat_p.device)
+        self.has_buf = [False] * len(self.params)       # momentum buffer initialised (torch: state['momentum_buffer'])
+
     def _runs(self, live):
         """Maximal contiguous ranges of the bucket whose parameters are live and share the first-step flag."""
         runs = []
@@ -104,9 +115,6 @@ class FlatSGD:
                            self.buf.data_ptr() + o * esz, k, self.lr, self.momentum, self.dampening, self.weight_decay,
                            int(self.nesterov), 1.0, int(first), stream())
         self.steps += 1
-
-    def set_lr(self, lr):
-        self.lr = float(lr)
 
     # ---- torch.optim.SGD-shaped state (job_runner.py:341 saves optimizer.state_dict() under "optimizer_dict")
     def state_dict(self):
@@ -136,6 +144,109 @@ class FlatSGD:
             self.buf[o:o + k].copy_(mb.reshape(-1).to(self.buf.device, torch.float32))
             self.has_buf[i] = True
         self.steps = int(sd.get("steps", max(self.steps, 1 if any(self.has_buf) else 0)))
+
+
+class FlatAdam(_FlatBucket):
+    """torch.optim.Adam semantics (betas, eps, weight_decay, amsgrad, maximize), or torch.optim.AdamW with
+    ``decoupled=True``, over the flat bucket (``spgnn_adam_step``).  As in torch, every parameter has its own step
+    count and a parameter whose ``grad`` is None is skipped: its count does not advance and no decay is applied.
+    The counts (``step_t``, int64 per parameter) live in device memory and the kernel advances them, so a
+    GraphedTrainStep replay takes the bias corrections of the step it really is.  A step is two launches whatever
+    the number of parameters: the count increment and one update over a device table of chunks of the live
+    parameters, built once per set of live parameters and kept (a captured graph may still read it)."""
+
+    CHUNK = 4096                                        # elements per block of the update kernel
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False,
+                 maximize=False, decoupled=False, process_group=None):
+        self.lr, self.betas, self.eps = float(lr), (float(betas[0]), float(betas[1])), float(eps)
+        self.weight_decay, self.amsgrad, self.maximize = float(weight_decay), bool(amsgrad), bool(maximize)
+        self.decoupled = bool(decoupled)
+        if not (self.lr >= 0.0 and self.eps >= 0.0 and self.weight_decay >= 0.0):         # torch's own checks
+            raise ValueError(f"Adam: lr, eps and weight_decay must be >= 0 (got {lr}, {eps}, {weight_decay})")
+        if not all(0.0 <= b < 1.0 for b in self.betas):
+            raise ValueError(f"Adam: betas must be in [0, 1) (got {betas})")
+        super().__init__(params, process_group)
+        dev = self.flat_p.device
+        self.exp_avg = torch.zeros(self.numel, dtype=torch.float32, device=dev)
+        self.exp_avg_sq = torch.zeros(self.numel, dtype=torch.float32, device=dev)
+        self.max_exp_avg_sq = torch.zeros_like(self.exp_avg) if self.amsgrad else None
+        self.step_t = torch.zeros(len(self.params), dtype=torch.int64, device=dev)
+        self._tables = {}
+
+    def _table(self, live):
+        """(int64 device tensor [chunks x {offset, length, parameter}, then the live indices], number of chunks)"""
+        key = tuple(live)
+        if key not in self._tables:
+            rows = []
+            for i in live:
+                o, k = self.offsets[i]
+                for c in range(0, k, self.CHUNK):
+                    rows += [o + c, min(self.CHUNK, k - c), i]
+            self._tables[key] = (torch.tensor(rows + list(live), dtype=torch.int64, device=self.flat_p.device),
+                                 len(rows) // 3)
+        return self._tables[key]
+
+    def step(self):
+        live = self._gather()
+        sdist.allreduce_sum_(self.flat_g, self.group)      # the ONE gradient collective of a step (no-op at world 1)
+        if live:
+            table, n_chunks = self._table(live)
+            lib().adam_step(ptr(self.flat_p), ptr(self.flat_g), ptr(self.exp_avg), ptr(self.exp_avg_sq),
+                            ptr(self.max_exp_avg_sq), ptr(self.step_t), ptr(table), n_chunks,
+                            table.data_ptr() + 8 * 3 * n_chunks, len(live), self.lr, self.betas[0], self.betas[1],
+                            self.eps, self.weight_decay, int(self.amsgrad), int(self.maximize), int(self.decoupled),
+                            stream())
+        self.steps += 1
+
+    # ---- the layout of torch.optim.Adam / AdamW.state_dict(), which job_runner.py saves under "optimizer_dict"
+    def _buffers(self):
+        names = [("exp_avg", self.exp_avg), ("exp_avg_sq", self.exp_avg_sq)]
+        return names + ([("max_exp_avg_sq", self.max_exp_avg_sq)] if self.amsgrad else [])
+
+    def state_dict(self):
+        counts = self.step_t.tolist()
+        state = {}
+        for i, (o, k) in enumerate(self.offsets):
+            if counts[i]:                               # torch creates a parameter's state at its first gradient
+                st = {"step": torch.tensor(float(counts[i]), dtype=torch.float32)}
+                for name, buf in self._buffers():
+                    st[name] = buf[o:o + k].view_as(self.params[i].data).detach().cpu().clone()
+                state[i] = st
+        group = dict(lr=self.lr, betas=self.betas, eps=self.eps, weight_decay=self.weight_decay, amsgrad=self.amsgrad,
+                     maximize=self.maximize, foreach=None, capturable=False, differentiable=False, fused=None,
+                     decoupled_weight_decay=self.decoupled, params=list(range(len(self.params))))
+        return {"state": state, "param_groups": [group], "steps": self.steps}
+
+    def load_state_dict(self, sd):
+        """A state dict of this class or of torch.optim.Adam / AdamW (CPU or CUDA tensors, ``step`` a tensor or a
+        number).  As in torch, the saved group's hyper-parameters replace the current ones."""
+        groups = sd["param_groups"]
+        if len(groups) != 1 or len(groups[0]["params"]) != len(self.params):
+            raise ValueError(f"FlatAdam: expected one parameter group of {len(self.params)} parameters")
+        group = groups[0]
+        self.lr = float(group.get("lr", self.lr))
+        self.betas = tuple(float(b) for b in group.get("betas", self.betas))
+        self.eps = float(group.get("eps", self.eps))
+        self.weight_decay = float(group.get("weight_decay", self.weight_decay))
+        self.amsgrad = bool(group.get("amsgrad", self.amsgrad))
+        self.maximize = bool(group.get("maximize", self.maximize))
+        self.decoupled = bool(group.get("decoupled_weight_decay", self.decoupled))
+        self.max_exp_avg_sq = torch.zeros_like(self.exp_avg) if self.amsgrad else None
+        self.exp_avg.zero_()
+        self.exp_avg_sq.zero_()
+        counts = [0] * len(self.params)
+        for i, st in sd.get("state", {}).items():
+            i = int(i)
+            o, k = self.offsets[i]
+            for name, buf in self._buffers():
+                t = st[name]
+                if t.numel() != k:
+                    raise ValueError(f"FlatAdam: state {i} '{name}' has {t.numel()} elements, the parameter {k}")
+                buf[o:o + k].copy_(t.reshape(-1).to(buf.device, torch.float32))
+            counts[i] = int(round(float(st["step"])))
+        self.step_t.copy_(torch.tensor(counts, dtype=torch.int64))
+        self.steps = int(sd.get("steps", max(counts)))
 
 
 def _allreduce_sums(group=None):
@@ -168,8 +279,9 @@ class GraphedTrainStep:
     each: the GPU waits for the host.  The step is captured once per batch and replayed: the learning rate, the
     momentum-buffer state and every pointer are frozen in the graph, the dropout / sampling masks are NOT — the first
     nodes of the graph bump a device-side step counter and copy it into the library's seed salt
-    (``spgnn_seed_salt_set``), so replay k draws the masks of seed + k.  ``loss`` is a device tensor refreshed by every
-    replay.  Re-capture (a new object) when the batch or the learning rate changes; world_size > 1 stays eager."""
+    (``spgnn_seed_salt_set``), so replay k draws the masks of seed + k.  FlatAdam's step counts (its bias corrections)
+    are not frozen either: they live in device memory and its kernel advances them.  ``loss`` is a device tensor
+    refreshed by every replay.  Re-capture (a new object) when the batch or the learning rate changes; world_size > 1 stays eager."""
 
     def __init__(self, net, g, opt, class_w, sampling_rate, warmup=3, group=None):
         if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
