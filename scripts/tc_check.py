@@ -30,7 +30,7 @@ def check(M, K1, K2, N, seed=0):
     return max(e_f, e_x, e_w)
 
 if __name__ == "__main__":
-    print(torch.cuda.get_device_name(0), "SPGNN_TN_SWAP=", os.environ.get("SPGNN_TN_SWAP"))
+    print(torch.cuda.get_device_name(0))
     worst = 0
     for shp in [(128, 64, 0, 16), (300, 64, 0, 48), (1000, 1024, 39, 130), (257, 39, 0, 258), (513, 100, 8, 22),
                 (5000, 1024, 40, 1028), (4096, 192, 0, 4100), (3001, 768, 0, 516)]:

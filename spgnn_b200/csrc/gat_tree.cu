@@ -329,10 +329,10 @@ __device__ __forceinline__ float4 act_slope4(float4 p, int act) {
 
 // NG gradient sources; ACT: activation known at compile time (0 = read it from the arguments); THREADS / 8 nodes are
 // taken per round and a slice takes KPER rounds; PF: how many rounds ahead a node's own-row operands (residual
-// projection, gradient sources) are loaded into registers.  PF == KPER is the first generation of this kernel
-// (512 threads, everything of the next slice loaded a whole slice ahead: 4 * KPER * (1 + NG) registers, which pinned
-// the kernel at 128 registers x 16 warps); PF = 2 with 896 threads keeps 8 * (1 + NG) prefetch registers and lets
-// 28 warps share the issue slots (the ncu source view showed neither DRAM nor issue slots saturated at 16 warps).
+// projection, gradient sources) are loaded into registers.  Loading a whole slice ahead (PF == KPER, the first
+// version of this kernel: 4 * KPER * (1 + NG) registers) pinned it at 128 registers x 16 warps; a shallower ring
+// keeps 4 * PF * (1 + NG) prefetch registers and lets more warps share the issue slots (the ncu source view showed
+// neither DRAM nor issue slots saturated at 16 warps).  Launch shapes: launch_bwd_act.
 template <int NG, int ACT, int THREADS, int KPER, int PF>
 __global__ void __launch_bounds__(THREADS, 1) gat_tree_bwd_kernel(const __grid_constant__ CUtensorMap zmap, const TArgs t) {
     constexpr int kThreads = THREADS, kQW = THREADS / 8;
@@ -670,25 +670,11 @@ static int launch_fwd_cfg(const CUtensorMap& zmap, TArgs& t, const Args& a, cons
 
 // Launch shape of the forward: 512 threads x 5-6 rounds of 64 nodes.  The shapes that help the backward (640 x 4,
 // 608 x 4, 896 x 3, 1024 x 3) measured within noise or slower here (0.91 - 0.95 vs 0.92 - 1.04 ms per launch,
-// profiles/r02_tree_bwd_variants.txt); SPGNN_TREE_FWD=1 selects 896 x 3-4 for A/B runs.
-static int fwd_variant() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SPGNN_TREE_FWD");
-        v = (e && atoi(e) == 1) ? 1 : 0;
-    }
-    return v;
-}
-
+// profiles/r02_tree_bwd_variants.txt).
 template <int ACT>
 static int launch_fwd_act(const CUtensorMap& zmap, TArgs& t, const Args& a, const spgnn_gat_layer* L, cudaStream_t st,
                           bool* handled) {
-    const int64_t n = L->max_nodes;
-    if (fwd_variant() == 1) {
-        if (n <= 3 * 112) return launch_fwd_cfg<ACT, 896, 3>(zmap, t, a, L, st, handled);
-        return launch_fwd_cfg<ACT, 896, 4>(zmap, t, a, L, st, handled);
-    }
-    if (n <= 5 * 64) return launch_fwd_cfg<ACT, 512, 5>(zmap, t, a, L, st, handled);
+    if (L->max_nodes <= 5 * 64) return launch_fwd_cfg<ACT, 512, 5>(zmap, t, a, L, st, handled);
     return launch_fwd_cfg<ACT, 512, 6>(zmap, t, a, L, st, handled);
 }
 
@@ -740,35 +726,11 @@ static int launch_bwd_cfg(const CUtensorMap& zmap, TArgs& t, const Args& a, cons
 //   640 x 4, 2 rounds ahead 1.83 - 1.88   |  640 x 4, whole-slice 1.98 - 2.01  |  608 x 4 1.93  |  832 x 3 1.93
 //   896 x 3 1.95 - 1.98  |  1024 x 3 (64 registers) 2.10 - 2.14: more warps do not help, the rounds of a slice must
 //   divide the tree evenly (301 = 80 + 80 + 80 + 61) because every slice ends in a block barrier.
-// SPGNN_TREE_BWD = 0 (first generation) / 1 (896 x 3) / 9 (640 x 4, 2 rounds ahead) keep the alternatives reachable.
-static int bwd_variant() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SPGNN_TREE_BWD");
-        v = e ? atoi(e) : 3;
-        if (v != 0 && v != 1 && v != 9) v = 3;
-    }
-    return v;
-}
-
 template <int NG, int ACT>
 static int launch_bwd_act(const CUtensorMap& zmap, TArgs& t, const Args& a, const spgnn_gat_layer* L, cudaStream_t st,
                           bool* handled) {
-    const int64_t n = L->max_nodes;
-    switch (bwd_variant()) {
-        case 0:
-            if (n <= 5 * 64) return launch_bwd_cfg<NG, ACT, 512, 5, 5>(zmap, t, a, L, st, handled);
-            return launch_bwd_cfg<NG, ACT, 512, 6, 6>(zmap, t, a, L, st, handled);
-        case 1:
-            if (n <= 3 * 112) return launch_bwd_cfg<NG, ACT, 896, 3, 2>(zmap, t, a, L, st, handled);
-            return launch_bwd_cfg<NG, ACT, 896, 4, 2>(zmap, t, a, L, st, handled);
-        case 9:
-            if (n <= 4 * 80) return launch_bwd_cfg<NG, ACT, 640, 4, 2>(zmap, t, a, L, st, handled);
-            return launch_bwd_cfg<NG, ACT, 640, 5, 2>(zmap, t, a, L, st, handled);
-        default:
-            if (n <= 4 * 80) return launch_bwd_cfg<NG, ACT, 640, 4, 3>(zmap, t, a, L, st, handled);
-            return launch_bwd_cfg<NG, ACT, 640, 5, 2>(zmap, t, a, L, st, handled);
-    }
+    if (L->max_nodes <= 4 * 80) return launch_bwd_cfg<NG, ACT, 640, 4, 3>(zmap, t, a, L, st, handled);
+    return launch_bwd_cfg<NG, ACT, 640, 5, 2>(zmap, t, a, L, st, handled);
 }
 
 int launch_bwd(const Args& a, const spgnn_gat_layer* L, cudaStream_t st, bool* handled) {

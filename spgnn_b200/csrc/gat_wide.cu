@@ -467,9 +467,10 @@ using namespace spgnn::wide;
 extern "C" int64_t spgnn_gat_wide_sizeof(void) { return (int64_t)sizeof(spgnn_gat_wide); }
 
 // NCH = four-column chunks per row: 16 lanes per node when that fills every pass of the chunk loop and 32 would not
+// (profiles/r02_aggx_lanes_per_node.txt)
 #define WIDE_DISPATCH_H(KERNEL, HH, NCH, ...)                                                   \
     do {                                                                                        \
-        if ((NCH) % 32 != 0 && (NCH) % 16 == 0 && wide_lanes_per_node() != 32)                  \
+        if ((NCH) % 32 != 0 && (NCH) % 16 == 0)                                                 \
             KERNEL<HH, 16><<<grid, kThreads, smem, st>>>(__VA_ARGS__);                          \
         else KERNEL<HH, 32><<<grid, kThreads, smem, st>>>(__VA_ARGS__);                         \
     } while (0)
@@ -480,15 +481,6 @@ extern "C" int64_t spgnn_gat_wide_sizeof(void) { return (int64_t)sizeof(spgnn_ga
         else WIDE_DISPATCH_H(KERNEL, 4, NCH, __VA_ARGS__);                  \
         SPGNN_LAUNCH_OK();                                                  \
     } while (0)
-// SPGNN_AGGX_LANES=32 forces one warp per node (A/B runs)
-static int wide_lanes_per_node() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SPGNN_AGGX_LANES");
-        v = (e && atoi(e) == 32) ? 32 : 16;
-    }
-    return v;
-}
 
 extern "C" int spgnn_gat_aggx_fwd(const spgnn_gat_wide* L, void* stream) {
     WArgs a{};

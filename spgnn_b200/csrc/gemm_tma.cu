@@ -141,12 +141,6 @@ __device__ __forceinline__ void nt_epilogue_tile(const NtArgs& g, uint32_t stg, 
     }
 }
 
-// CL = 2: clusters of two CTAs work on two adjacent m-tiles of the SAME n-tile in lock step; each CTA fetches half of
-// the weight tile and multicasts it to both, so the B tile crosses the L2 -> SM fabric once per cluster.  The ncu
-// capture of the CL = 1 kernel (profiles/r01_ncu_full_step_79ms_*) shows the big projections bound by that fabric
-// (85 KB per k-block per SM against ~43 B/clk/SM), tensor pipe 65-76 % busy.  Stage s of BOTH CTAs is free once both
-// UMMA issuers have committed it (empty barriers count CL arrivals, commits are multicast).
-template <int CL>
 __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_constant__ NtMaps maps, const NtArgs g) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -158,7 +152,7 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
     if (threadIdx.x == 0) {
         for (int s = 0; s < g.stages; ++s) {
             mbar_init(smem_u32(&sh->full[s]), 1);
-            mbar_init(smem_u32(&sh->empty[s]), CL);
+            mbar_init(smem_u32(&sh->empty[s]), 1);
         }
         for (int b = 0; b < 2; ++b) {
             mbar_init(smem_u32(&sh->tmem_full[b]), 1);
@@ -174,15 +168,11 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
     if (warp == kEpiWarps) tmem_alloc(smem_u32(&sh->tmem_base), 512);
     tc_fence_before();
     __syncthreads();
-    if (CL > 1) cluster_sync_all();          // the peer's barriers exist before anything is multicast into them
     tc_fence_after();
     const uint32_t tmem_base = sh->tmem_base;
 
-    // work items: (m-tile, n-tile) for CL = 1; (pair of m-tiles, n-tile) per cluster for CL = 2, this CTA takes
-    // m-tile 2 * pair + rank (a pair's second tile may lie beyond M: loads are zero-filled, nothing is stored)
-    const int rank = CL > 1 ? (int)cluster_ctarank() : 0;
-    const int64_t n_tiles = (CL > 1 ? (g.nt_m + CL - 1) / CL : g.nt_m) * g.nt_n;
-    const int64_t tile0 = blockIdx.x / CL, tile_step = gridDim.x / CL;
+    const int64_t n_tiles = g.nt_m * g.nt_n;
+    const int64_t tile0 = blockIdx.x, tile_step = gridDim.x;
     const int nkb = g.kb1 + g.kb2;
 
     if (warp < kEpiWarps) {
@@ -194,7 +184,7 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
         for (int64_t tile = tile0; tile < n_tiles; tile += tile_step, ++it) {
             const int buf = it & 1;
             const uint32_t par = (it >> 1) & 1;
-            const int64_t m0 = ((tile / g.nt_n) * CL + rank) * BM;
+            const int64_t m0 = (tile / g.nt_n) * BM;
             const int n0 = (int)(tile % g.nt_n) * g.BN;
             const int ncols = min(g.BN, g.N - n0);
             mbar_wait(smem_u32(&sh->tmem_full[buf]), par);
@@ -240,9 +230,7 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
                             umma_bf16(tmem_d, dah, dbl, idesc, 1);
                             umma_bf16(tmem_d, dal, dbh, idesc, 1);
                         }
-                        // frees the smem stage when these UMMAs retire (in both CTAs of a cluster)
-                        if (CL > 1) umma_commit_mc(smem_u32(&sh->empty[s]), (uint16_t)((1u << CL) - 1));
-                        else umma_commit(smem_u32(&sh->empty[s]));
+                        umma_commit(smem_u32(&sh->empty[s]));          // frees the smem stage when these UMMAs retire
                     }
                     __syncwarp();
                 }
@@ -255,7 +243,7 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
         uint32_t kcount = 0;
         const uint32_t tx = (uint32_t)g.stage_bytes;
         for (int64_t tile = tile0; tile < n_tiles; tile += tile_step) {
-            const int m0 = (int)(((tile / g.nt_n) * CL + rank) * BM);
+            const int m0 = (int)((tile / g.nt_n) * BM);
             const int n0 = (int)(tile % g.nt_n) * g.BN;
             for (int kb = 0; kb < nkb; ++kb, ++kcount) {
                 const int s = kcount % g.stages;
@@ -266,23 +254,13 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
                 const uint32_t dst = smem_base + s * g.stage_bytes;
                 if (kb < g.kb1) tma_load_3d(dst, &maps.a1, bar, kb * BK, m0, 0);
                 else tma_load_3d(dst, &maps.a2, bar, (kb - g.kb1) * BK, m0, 0);
-                if (CL > 1) {
-                    // this CTA's half of the weight tile (rows [rank * BN/2, ...) of both planes) goes to both CTAs
-                    const int half = g.BN / CL;
-                    const uint32_t off = (uint32_t)(rank * half * 128);
-                    const uint16_t mask = (uint16_t)((1u << CL) - 1);
-                    tma_load_3d_mc(dst + kABytes + off, &maps.b, bar, kb * BK, n0 + rank * half, 0, mask);
-                    tma_load_3d_mc(dst + kABytes + g.BN * 128 + off, &maps.b, bar, kb * BK, n0 + rank * half, 1, mask);
-                } else {
-                    tma_load_3d(dst + kABytes, &maps.b, bar, kb * BK, n0, 0);
-                }
+                tma_load_3d(dst + kABytes, &maps.b, bar, kb * BK, n0, 0);
             }
         }
     }
 
     tc_fence_before();
     __syncthreads();
-    if (CL > 1) cluster_sync_all();          // no CTA leaves while its peer may still signal its barriers
     if (warp == kEpiWarps) {
         tc_fence_after();
         tmem_dealloc(tmem_base, 512);
@@ -295,7 +273,8 @@ __global__ void __launch_bounds__(kThreads, 1) nt_planes_kernel(const __grid_con
 // (k-step, pass) that reads both halves, and each CTA drains its own 128 accumulator lanes.  Per CTA and k-block that
 // is 32 KB + BN * 128 B through the L2 -> SM path instead of 32 KB + BN * 256 B: the chip-wide L2 throughput
 // (~6300 B/clk = 42.6 B/clk/SM) is what bounds the single-CTA kernel on the big projections (tensor pipe 62 - 73 %),
-// and TMA multicast does not relieve it at cluster size 2 (nt_planes_kernel<2>, measured neutral).
+// and TMA multicast of the weight tile did not relieve it at cluster size 2 (measured neutral and removed,
+// profiles/r01_gemm_check_cluster_vs_plain.txt).
 // Barriers: full[s] of the LEADER collects the transaction bytes of both CTAs' loads (cp.async.bulk.tensor
 // .cta_group::2 signals the peer's barrier); empty[s] / tmem_full[b] are arrived in both CTAs by multicast commits;
 // tmem_empty[b] of the leader counts the epilogue threads of both CTAs (the peer arrives through the cluster window).
@@ -746,150 +725,6 @@ __global__ void __launch_bounds__(kWideThreads, 1) wide_kernel(const __grid_cons
     }
 }
 
-// The wide kernel on CTA pairs (see nt_pair_kernel): a pair owns 256 rows x BN columns x H heads; each CTA loads its A
-// tile and HALF of every weight tile (48 instead of 64 KB per k-block at BN = 128).  Opt-in: measured slower than the
-// single-CTA kernel at the bench size (see spgnn_wide_linear).
-__global__ void __launch_bounds__(kWideThreads, 1) wide_pair_kernel(const __grid_constant__ WideMaps maps, const WideArgs g) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    const int stages_bytes = g.stages * g.stage_bytes;
-    NtShared* sh = reinterpret_cast<NtShared*>(smem + stages_bytes);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t smem_base = smem_u32(smem);
-    const uint32_t rank = cluster_ctarank();
-    const bool leader = rank == 0;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < g.stages; ++s) {
-            mbar_init(smem_u32(&sh->full[s]), 1);
-            mbar_init(smem_u32(&sh->empty[s]), 1);
-        }
-        for (int b = 0; b < 2; ++b) {
-            mbar_init(smem_u32(&sh->tmem_full[b]), 1);
-            mbar_init(smem_u32(&sh->tmem_empty[b]), 2 * kWideEpiWarps);
-        }
-        fence_barrier_init();
-    }
-    if (warp == kWideEpiWarps + 1 && lane == 0) {
-        prefetch_tmap(&maps.a);
-        prefetch_tmap(&maps.b);
-    }
-    if (warp == kWideEpiWarps) tmem_alloc_pair(smem_u32(&sh->tmem_base), 512);
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();
-    tc_fence_after();
-    const uint32_t tmem_base = sh->tmem_base;
-
-    const int64_t n_tiles = ((g.nt_m + 1) / 2) * g.nt_n;
-    const int64_t tile0 = blockIdx.x / 2, tile_step = gridDim.x / 2;
-    const int nkb = g.nparts * g.kbp;                // k-blocks per head
-    const int accw = g.H * g.BN;                     // TMEM columns per accumulator buffer
-    const int half = g.BN / 2;
-
-    if (warp < kWideEpiWarps) {
-        // ===================================================== epilogue (both CTAs)
-        int it = 0;
-        const uint32_t stg = smem_base + stages_bytes + 256 + warp * (32 * 16 * 4);
-        float* dbias_row = g.dbias_ws ? g.dbias_ws + (int64_t)blockIdx.x * (g.H * g.F) : nullptr;
-        const uint32_t empty_leader0 = mapa_u32(smem_u32(&sh->tmem_empty[0]), 0);
-        const uint32_t empty_leader1 = mapa_u32(smem_u32(&sh->tmem_empty[1]), 0);
-        for (int64_t tile = tile0; tile < n_tiles; tile += tile_step, ++it) {
-            const int buf = it & 1;
-            const uint32_t par = (it >> 1) & 1;
-            const int64_t m0 = ((tile / g.nt_n) * 2 + rank) * BM;
-            const int n0 = (int)(tile % g.nt_n) * g.BN;
-            const int ncols = min(g.BN, g.F - n0);
-            const uint32_t taddr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(buf * accw);
-            const uint32_t fb = smem_u32(&sh->tmem_full[buf]);
-            if (g.mode == 0) {
-                if (g.act == SPGNN_ACT_ELU) wide_epilogue_tile<SPGNN_ACT_ELU, 0>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else if (g.act == SPGNN_ACT_NONE) wide_epilogue_tile<SPGNN_ACT_NONE, 0>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else wide_epilogue_tile<-1, 0>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-            } else {
-                if (g.act == SPGNN_ACT_ELU) wide_epilogue_tile<SPGNN_ACT_ELU, 1>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else if (g.act == SPGNN_ACT_NONE) wide_epilogue_tile<SPGNN_ACT_NONE, 1>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else wide_epilogue_tile<-1, 1>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(buf ? empty_leader1 : empty_leader0);
-        }
-    } else if (warp == kWideEpiWarps) {
-        // ===================================================== UMMA issuer (leader; whole warp in the loop, one lane issues)
-        if (leader) {
-            int it = 0;
-            uint32_t kcount = 0;
-            const uint32_t idesc = make_idesc_pair(g.BN);
-            const uint32_t tbase = __shfl_sync(kFull, tmem_base, 0);
-            for (int64_t tile = tile0; tile < n_tiles; tile += tile_step, ++it) {
-                const int buf = it & 1;
-                const uint32_t par = (it >> 1) & 1;
-                mbar_wait(smem_u32(&sh->tmem_empty[buf]), par ^ 1);
-                tc_fence_after();
-                for (int h = 0; h < g.H; ++h) {
-                    const uint32_t tmem_d = tbase + (uint32_t)(buf * accw + h * g.BN);
-                    for (int kb = 0; kb < nkb; ++kb, ++kcount) {
-                        const int s = kcount % g.stages;
-                        const uint32_t sp = (kcount / g.stages) & 1;
-                        mbar_wait(smem_u32(&sh->full[s]), sp);
-                        tc_fence_after();
-                        const uint32_t a_hi = smem_base + s * g.stage_bytes;
-                        const uint32_t a_lo = a_hi + BM * 128;
-                        const uint32_t b_hi = a_hi + kABytes;
-                        const uint32_t b_lo = b_hi + half * 128;
-                        if (elect_one()) {
-#pragma unroll
-                            for (int k = 0; k < BK / 16; ++k) {
-                                const uint32_t ko = k * 32;
-                                const uint64_t dah = make_desc(a_hi + ko, 16, 1024), dal = make_desc(a_lo + ko, 16, 1024);
-                                const uint64_t dbh = make_desc(b_hi + ko, 16, 1024), dbl = make_desc(b_lo + ko, 16, 1024);
-                                umma_bf16_pair(tmem_d, dah, dbh, idesc, (kb | k) != 0);
-                                umma_bf16_pair(tmem_d, dah, dbl, idesc, 1);
-                                umma_bf16_pair(tmem_d, dal, dbh, idesc, 1);
-                            }
-                            umma_commit_pair(smem_u32(&sh->empty[s]), 3);
-                        }
-                        __syncwarp();
-                    }
-                }
-                if (elect_one()) umma_commit_pair(smem_u32(&sh->tmem_full[buf]), 3);
-                __syncwarp();
-            }
-        }
-    } else if (lane == 0) {
-        // ===================================================== TMA producer (one thread per CTA)
-        uint32_t kcount = 0;
-        const uint32_t tx = 2u * (uint32_t)g.stage_bytes;
-        for (int64_t tile = tile0; tile < n_tiles; tile += tile_step) {
-            const int m0 = (int)(((tile / g.nt_n) * 2 + rank) * BM);
-            const int n0 = (int)(tile % g.nt_n) * g.BN + (int)rank * half;
-            for (int h = 0; h < g.H; ++h) {
-                for (int kb = 0; kb < nkb; ++kb, ++kcount) {
-                    const int s = kcount % g.stages;
-                    const uint32_t sp = (kcount / g.stages) & 1;
-                    mbar_wait(smem_u32(&sh->empty[s]), sp ^ 1);
-                    const uint32_t bar = mapa_u32(smem_u32(&sh->full[s]), 0);
-                    if (leader) mbar_expect_tx(smem_u32(&sh->full[s]), tx);
-                    const uint32_t dst = smem_base + s * g.stage_bytes;
-                    const int part = kb / g.kbp, j = kb - part * g.kbp;
-                    const int acol = (part == 0 ? h : g.H) * g.kp + j * BK;
-                    tma_load_3d_pair(dst, &maps.a, bar, acol, m0, 0);
-                    tma_load_3d_pair(dst + kABytes, &maps.b, bar, kb * BK, h * g.F + n0, 0);
-                }
-            }
-        }
-    }
-
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();
-    if (warp == kWideEpiWarps) {
-        tc_fence_after();
-        tmem_dealloc_pair(tmem_base, 512);
-    }
-}
-
 __global__ void wide_dbias_reduce_kernel(const float* __restrict__ part, int64_t nparts, int64_t HF, float* __restrict__ out) {
     for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < HF; c += (int64_t)gridDim.x * blockDim.x) {
         float s = 0.f;
@@ -1193,7 +1028,7 @@ static EncodeTiledFn encode_fn() {
 
 // planes [rows, cols] (ld elements between rows, ps elements between the hi and lo plane) -> 3-D map {cols, rows, 2}
 static int make_planes_map(CUtensorMap* m, const void* hi, int64_t rows, int64_t cols, int64_t ld, int64_t ps,
-                           int box_cols, int box_rows, int box_planes = 2) {
+                           int box_cols, int box_rows) {
     EncodeTiledFn fn = encode_fn();
     SPGNN_REQUIRE(fn, "cuTensorMapEncodeTiled is not available from the driver");
     SPGNN_REQUIRE(((uintptr_t)hi & 15) == 0 && (ld * 2) % 16 == 0 && (ps * 2) % 16 == 0 && rows > 0 && cols > 0,
@@ -1201,7 +1036,7 @@ static int make_planes_map(CUtensorMap* m, const void* hi, int64_t rows, int64_t
                   (long long)ld, (long long)ps);
     cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, 2};
     cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)ps * 2};
-    cuuint32_t box[3] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, (cuuint32_t)box_planes};
+    cuuint32_t box[3] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, 2};
     cuuint32_t es[3] = {1, 1, 1};
     CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(hi), dims, strides, box, es,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -1225,30 +1060,28 @@ static unsigned split_grid(int64_t total) {
     return (unsigned)(want < cap ? want : cap);
 }
 
-// Co-resident 2-CTA clusters of a pair kernel on the CURRENT device (0: cluster launches unavailable / disabled).  Cached
-// per device ordinal: the dynamic-shared-memory opt-in and the occupancy are per-device properties.
-template <typename Kernel>
-static int pair_clusters_of(Kernel kernel, int threads, const char* env, bool default_on, int* cache /* [64], -1 */) {
+// Co-resident 2-CTA clusters of nt_pair_kernel on the CURRENT device (0: cluster launches unavailable).  Cached per
+// device ordinal: the dynamic-shared-memory opt-in and the occupancy are per-device properties.
+static int nt_pair_clusters() {
+    struct Cache { int v[64]; Cache() { for (int& x : v) x = -1; } };
+    static Cache cache;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
-    if (cache[dev] >= 0) return cache[dev];
+    if (cache.v[dev] >= 0) return cache.v[dev];
     int n = 0;
-    const char* e = getenv(env);
-    const bool on = e ? atoi(e) != 0 : default_on;
-    if (on && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit) == cudaSuccess) {
+    if (cudaFuncSetAttribute(nt_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit) == cudaSuccess) {
         cudaLaunchConfig_t cfg{};
         cudaLaunchAttribute at[1];
         at[0].id = cudaLaunchAttributeClusterDimension;
         at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.gridDim = dim3((unsigned)(sm_count() / 2 * 2)); cfg.blockDim = dim3((unsigned)threads);
+        cfg.gridDim = dim3((unsigned)(sm_count() / 2 * 2)); cfg.blockDim = dim3(kThreads);
         cfg.dynamicSmemBytes = kSmemLimit; cfg.attrs = at; cfg.numAttrs = 1;
-        if (cudaOccupancyMaxActiveClusters(&n, kernel, &cfg) != cudaSuccess) n = 0;
+        if (cudaOccupancyMaxActiveClusters(&n, nt_pair_kernel, &cfg) != cudaSuccess) n = 0;
     }
     (void)cudaGetLastError();
-    cache[dev] = n;
+    cache.v[dev] = n;
     return n;
 }
-struct PairCache { int v[64]; PairCache() { for (int& x : v) x = -1; } };
 
 // C = [A1|A2] * Bplanes^T with Bplanes [N, ldb] already split (hi at Bhi, lo at Bhi + N*ldb)
 static int launch_nt(const __nv_bfloat16* A1, int64_t lda1, int64_t ps1, int64_t K1, const __nv_bfloat16* A2,
@@ -1256,58 +1089,43 @@ static int launch_nt(const __nv_bfloat16* A1, int64_t lda1, int64_t ps1, int64_t
                      int act, float slope, float* C, int64_t ldc, int64_t M, int64_t N, cudaStream_t st,
                      float mask_p = 0.f, uint64_t mask_seed = 0, int64_t mask_chunks = 0, int64_t mask_chunk_off = 0) {
     static DeviceOnce attr;
-    static int max_clusters = 0;             // co-resident 2-CTA clusters (0: cluster launches unavailable)
     if (attr.pending()) {
-        SPGNN_CUDA_OK(cudaFuncSetAttribute(nt_planes_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
-        SPGNN_CUDA_OK(cudaFuncSetAttribute(nt_planes_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
-        // opt-in: measured neutral on B200 (profiles/r01_gemm_check_cluster_vs_plain.txt) - the projections are
-        // limited by board power (sw_power_cap, SM clock 1.3-1.7 GHz under the 3-pass UMMA load), not by the fabric
-        const char* e = getenv("SPGNN_NT_CLUSTER");
-        if (e && atoi(e) == 2) {
-            cudaLaunchConfig_t cfg{};
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension;
-            at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-            cfg.gridDim = dim3((unsigned)(sm_count() / 2 * 2)); cfg.blockDim = dim3(kThreads);
-            cfg.dynamicSmemBytes = kSmemLimit; cfg.attrs = at; cfg.numAttrs = 1;
-            int n = 0;
-            if (cudaOccupancyMaxActiveClusters(&n, nt_planes_kernel<2>, &cfg) == cudaSuccess) max_clusters = n;
-            else (void)cudaGetLastError();
-        }
+        SPGNN_CUDA_OK(cudaFuncSetAttribute(nt_planes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
         attr.done();
     }
     NtMaps maps;
     NtArgs a{};
     pick_bn((int)N, &a.BN, &a.nt_n);
-    // CTA pairs (cta_group::2) unless SPGNN_NT_PAIR=0
-    static PairCache pair_cache;
-    const int pair_clusters = pair_clusters_of(nt_pair_kernel, kThreads, "SPGNN_NT_PAIR", true, pair_cache.v);
-    // Measured on 1.23 M rows (profiles/r02_nt_pair_vs_single.txt): gat0 / gat1 forward -6..-12 % / -19..-25 %, dX of
-    // gat1 / the output layer (K = 4100 -> 192 columns) -17..-21 % / -28 %; output-bound shapes (small K: pgnn0-2,
-    // K = 192 -> 4100 columns) lose 10 - 30 % to the coupling of the two epilogues and stay on the single-CTA kernel
+    // CTA pairs (cta_group::2), measured on 1.23 M rows (profiles/r02_nt_pair_vs_single.txt): gat0 / gat1 forward
+    // -6..-12 % / -19..-25 %, dX of gat1 / the output layer (K = 4100 -> 192 columns) -17..-21 % / -28 %; output-bound
+    // shapes (small K: pgnn0-2, K = 192 -> 4100 columns) lose 10 - 30 % to the coupling of the two epilogues and stay
+    // on the single-CTA kernel
+    const int pair_clusters = nt_pair_clusters();
     const int64_t Kt = K1 + K2;
-    if (pair_clusters > 0 && Kt >= 256 && (N >= 320 || Kt >= 512) && N >= 64 &&
-        ceil_div(M, BM) >= 4 * (int64_t)pair_clusters) {
-        int rc = make_planes_map(&maps.a1, A1, M, K1, lda1, ps1, BK, BM);
+    const bool pair = pair_clusters > 0 && Kt >= 256 && (N >= 320 || Kt >= 512) && N >= 64 &&
+                      ceil_div(M, BM) >= 4 * (int64_t)pair_clusters;
+    int rc = make_planes_map(&maps.a1, A1, M, K1, lda1, ps1, BK, BM);
+    if (rc) return rc;
+    if (A2 && K2 > 0) {
+        rc = make_planes_map(&maps.a2, A2, M, K2, lda2, ps2, BK, BM);
         if (rc) return rc;
-        if (A2 && K2 > 0) {
-            rc = make_planes_map(&maps.a2, A2, M, K2, lda2, ps2, BK, BM);
-            if (rc) return rc;
-        } else {
-            maps.a2 = maps.a1;
-        }
-        rc = make_planes_map(&maps.b, Bhi, N, ldb, ldb, N * ldb, BK, a.BN / 2);
-        if (rc) return rc;
-        a.bias = bias; a.act = act; a.slope = slope; a.C = C; a.ldc = ldc; a.M = M; a.N = (int)N;
-        a.mthr = mask_p > 0.f ? (uint32_t)(mask_p * 65536.f + 0.5f) : 0u;
-        a.mscale = mask_p > 0.f ? 1.f / (1.f - mask_p) : 1.f;
-        a.mseed = mask_seed; a.mnch = mask_chunks > 0 ? mask_chunks : (N + 3) / 4; a.moff = mask_chunk_off;
-        a.nt_m = ceil_div(M, BM);
-        a.kb1 = (int)ceil_div(K1, BK);
-        a.kb2 = (A2 && K2 > 0) ? (int)ceil_div(K2, BK) : 0;
-        a.stage_bytes = kABytes + a.BN * 128;           // this CTA's A tile + its half of the weight tile
-        a.stages = (kSmemLimit - kNtFixed) / a.stage_bytes;
-        if (a.stages > kMaxStages) a.stages = kMaxStages;
+    } else {
+        maps.a2 = maps.a1;
+    }
+    // each CTA of a pair loads half of the weight tile
+    rc = make_planes_map(&maps.b, Bhi, N, ldb, ldb, N * ldb, BK, pair ? a.BN / 2 : a.BN);
+    if (rc) return rc;
+    a.bias = bias; a.act = act; a.slope = slope; a.C = C; a.ldc = ldc; a.M = M; a.N = (int)N;
+    a.mthr = mask_p > 0.f ? (uint32_t)(mask_p * 65536.f + 0.5f) : 0u;
+    a.mscale = mask_p > 0.f ? 1.f / (1.f - mask_p) : 1.f;
+    a.mseed = mask_seed; a.mnch = mask_chunks > 0 ? mask_chunks : (N + 3) / 4; a.moff = mask_chunk_off;
+    a.nt_m = ceil_div(M, BM);
+    a.kb1 = (int)ceil_div(K1, BK);
+    a.kb2 = (A2 && K2 > 0) ? (int)ceil_div(K2, BK) : 0;
+    a.stage_bytes = kABytes + a.BN * (pair ? 128 : 256);
+    a.stages = (kSmemLimit - kNtFixed) / a.stage_bytes;
+    if (a.stages > kMaxStages) a.stages = kMaxStages;
+    if (pair) {
         const int64_t items = ceil_div(a.nt_m, 2) * a.nt_n;
         cudaLaunchConfig_t cfg{};
         cudaLaunchAttribute at[1];
@@ -1320,45 +1138,9 @@ static int launch_nt(const __nv_bfloat16* A1, int64_t lda1, int64_t ps1, int64_t
         count_launch();
         return SPGNN_OK;
     }
-    // clusters pay when several m-tiles share a weight tile that is worth a k-loop: not for skinny outputs
-    const bool cluster = max_clusters > 0 && ceil_div(M, BM) >= 4 * (int64_t)max_clusters && a.BN >= 64;
-    int rc = make_planes_map(&maps.a1, A1, M, K1, lda1, ps1, BK, BM);
-    if (rc) return rc;
-    if (A2 && K2 > 0) {
-        rc = make_planes_map(&maps.a2, A2, M, K2, lda2, ps2, BK, BM);
-        if (rc) return rc;
-    } else {
-        maps.a2 = maps.a1;
-    }
-    rc = cluster ? make_planes_map(&maps.b, Bhi, N, ldb, ldb, N * ldb, BK, a.BN / 2, 1)
-                 : make_planes_map(&maps.b, Bhi, N, ldb, ldb, N * ldb, BK, a.BN);
-    if (rc) return rc;
-    a.bias = bias; a.act = act; a.slope = slope; a.C = C; a.ldc = ldc; a.M = M; a.N = (int)N;
-    a.mthr = mask_p > 0.f ? (uint32_t)(mask_p * 65536.f + 0.5f) : 0u;
-    a.mscale = mask_p > 0.f ? 1.f / (1.f - mask_p) : 1.f;
-    a.mseed = mask_seed; a.mnch = mask_chunks > 0 ? mask_chunks : (N + 3) / 4; a.moff = mask_chunk_off;
-    a.nt_m = ceil_div(M, BM);
-    a.kb1 = (int)ceil_div(K1, BK);
-    a.kb2 = (A2 && K2 > 0) ? (int)ceil_div(K2, BK) : 0;
-    a.stage_bytes = kABytes + a.BN * 256;
-    a.stages = (kSmemLimit - kNtFixed) / a.stage_bytes;
-    if (a.stages > kMaxStages) a.stages = kMaxStages;
-    if (cluster) {
-        const int64_t items = ceil_div(a.nt_m, 2) * a.nt_n;
-        cudaLaunchConfig_t cfg{};
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.gridDim = dim3((unsigned)(2 * (items < max_clusters ? items : max_clusters)));
-        cfg.blockDim = dim3(kThreads);
-        cfg.dynamicSmemBytes = kSmemLimit; cfg.stream = st; cfg.attrs = at; cfg.numAttrs = 1;
-        SPGNN_CUDA_OK(cudaLaunchKernelEx(&cfg, nt_planes_kernel<2>, maps, a));
-        count_launch();
-        return SPGNN_OK;
-    }
     const int64_t tiles = a.nt_m * a.nt_n;
     const unsigned grid = (unsigned)(tiles < sm_count() ? tiles : sm_count());
-    nt_planes_kernel<1><<<grid, kThreads, kSmemLimit, st>>>(maps, a);
+    nt_planes_kernel<<<grid, kThreads, kSmemLimit, st>>>(maps, a);
     SPGNN_LAUNCH_OK();
     return SPGNN_OK;
 }
@@ -1483,44 +1265,21 @@ extern "C" int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa,
     if (rc) return rc;
     rc = make_planes_map(&maps.b, hi, HF, ldb, ldb, HF * ldb, BK, a.BN);
     if (rc) return rc;
-    // CTA pairs (cta_group::2) are OPT-IN here (SPGNN_WIDE_PAIR=1): correct (scripts/wide_pair_probe.py), but slower at
-    // the bench size -- forward 5.71 -> 6.05 ms, backward 6.52 -> 7.54 ms (profiles/r02_wide_pair_probe.txt): with
-    // BN = 128 and a 16-warp epilogue per CTA the leader's wait for BOTH epilogues costs more than the halved weight
-    // traffic saves.  Needs F % BN == 0 (every CTA loads exactly half a weight tile) and enough m-tiles for every pair
-    static PairCache pair_cache;
-    const int pair_clusters = pair_clusters_of(wide_pair_kernel, kWideThreads, "SPGNN_WIDE_PAIR", false, pair_cache.v);
-    const bool pair = pair_clusters > 0 && F % a.BN == 0 && a.BN % 32 == 0 && a.nt_m >= 4 * (int64_t)pair_clusters;
-    if (pair) {
-        rc = make_planes_map(&maps.b, hi, HF, ldb, ldb, HF * ldb, BK, a.BN / 2);
-        if (rc) return rc;
-    }
-    a.stage_bytes = kABytes + a.BN * (pair ? 128 : 256);
-    const int fixed = kWideFixed;
-    a.stages = (kSmemLimit - fixed) / a.stage_bytes;
+    // A CTA-pair variant was slower at the bench size and was removed (profiles/r02_wide_pair_probe.txt).
+    a.stage_bytes = kABytes + a.BN * 256;
+    a.stages = (kSmemLimit - kWideFixed) / a.stage_bytes;
     if (a.stages > kMaxStages) a.stages = kMaxStages;
     SPGNN_REQUIRE(a.stages >= 2, "wide_linear: not enough shared memory for two pipeline stages");
-    const int64_t tiles = pair ? ceil_div(a.nt_m, 2) * a.nt_n : a.nt_m * a.nt_n;
-    const unsigned grid = pair ? (unsigned)(2 * (tiles < pair_clusters ? tiles : pair_clusters))
-                               : (unsigned)(tiles < sm_count() ? tiles : sm_count());
+    const int64_t tiles = a.nt_m * a.nt_n;
+    const unsigned grid = (unsigned)(tiles < sm_count() ? tiles : sm_count());
     float* part = nullptr;
     if (mode == 1 && dbias) {
         part = reinterpret_cast<float*>(((uintptr_t)(hi + 2 * HF * ldb) + 255) & ~(uintptr_t)255);
         a.dbias_ws = part;
         SPGNN_CUDA_OK(cudaMemsetAsync(part, 0, (size_t)grid * HF * sizeof(float), st));
     }
-    if (pair) {
-        cudaLaunchConfig_t cfg{};
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kWideThreads);
-        cfg.dynamicSmemBytes = kSmemLimit; cfg.stream = st; cfg.attrs = at; cfg.numAttrs = 1;
-        SPGNN_CUDA_OK(cudaLaunchKernelEx(&cfg, wide_pair_kernel, maps, a));
-        count_launch();
-    } else {
-        wide_kernel<<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
-        SPGNN_LAUNCH_OK();
-    }
+    wide_kernel<<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
+    SPGNN_LAUNCH_OK();
     if (part) {
         wide_dbias_reduce_kernel<<<(unsigned)ceil_div(HF, 128), 128, 0, st>>>(part, grid, HF, dbias);
         SPGNN_LAUNCH_OK();

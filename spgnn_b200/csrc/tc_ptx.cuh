@@ -47,16 +47,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, 
         : "memory");
 }
 
-// same, delivered to the same CTA-relative shared address (and signalled on the same CTA-relative mbarrier) of every
-// CTA of the cluster named in cta_mask: ONE read of L2 feeds several SMs
-__device__ __forceinline__ void tma_load_3d_mc(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2,
-                                               uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%4, %5, %6}], [%2], %3;" ::"r"(dst),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "h"(cta_mask), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
 // thread-block cluster helpers
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
@@ -99,13 +89,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
 // arrive on an mbarrier once every previously issued UMMA of this thread has completed
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// same, arriving on the mbarrier at this CTA-relative address in every CTA of cta_mask (a stage that a peer fills by
-// multicast is only free once BOTH CTAs' UMMAs have read it)
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(cta_mask)
-                 : "memory");
 }
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
     asm volatile(

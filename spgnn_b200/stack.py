@@ -16,7 +16,6 @@ PyTorch is plumbing here: memory, streams, the autograd hook-up of the parameter
 from __future__ import annotations
 
 import ctypes
-import os
 
 import torch
 from torch.autograd import Function
@@ -82,10 +81,6 @@ class _Wide(ctypes.Structure):
 WIDE_OUTPUT_LAYER = True
 # One CTA per graph with the graph's rows staged in shared memory (spgnn_gat_layer.node_off).  Off: chunk kernels.
 TREE_KERNELS = True
-# The feat_drop mask of a layer's input is applied to the gradient in that layer's dX GEMM epilogue (tensor-bound, idle
-# issue slots) instead of in the producing layer's aggregation backward (issue-bound: the mask hash was a quarter of
-# its destination-side instructions).  Off (SPGNN_FOLD_MASK=0): the aggregation backward masks its gradient sources.
-FOLD_MASK = os.environ.get("SPGNN_FOLD_MASK", "1") != "0"
 
 _checked = False
 
@@ -536,14 +531,16 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
         extra.setdefault(plan.outputs[0], []).append(planes_linear_bwd_input(glp, head[0], head[0].shape[1]))
         tape.emb_planes = None
     dX = {}             # layer index -> fp32 [N, k] gradient of its concatenated (dropped) input
-    masked = set()      # layers whose dX already includes their own feat_drop mask
+    # layers whose dX already includes their own feat_drop mask: the mask is applied in the dX GEMM epilogue
+    # (tensor-bound, idle issue slots) rather than in the producing layer's aggregation backward (issue-bound: the
+    # mask hash was a quarter of its destination-side instructions).  The aggregate-first backward's dX is unmasked.
+    masked = set()
     for i in range(nL - 1, -1, -1):
         L = plan.layers[i]
         conv = L.conv
         srcs = []
         for ci, off in plan.consumers.get(L.output, []):
             if ci in dX and dX[ci] is not None and off < dX[ci].shape[1]:
-                # a dX that came out of the masked dX GEMM below already carries layer ci's feat_drop mask
                 pm = 0.0 if ci in masked else tape.pdrop[ci]
                 srcs.append((dX[ci], off, pm, tape.fseed[ci], (plan.layers[ci].k_in + 3) // 4))
         for g in extra.get(L.output, []):
@@ -558,8 +555,9 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
         if isinstance(tape.layers[i], _WideRec):
             rec = tape.layers[i]
             tape.layers[i] = None
-            if any(p > 0.0 or off for _, off, p, _, _ in srcs):
-                raise SpgnnError("stack: a head-averaged output layer cannot have masked gradient sources")
+            # every consumer of an aggregate-first layer has no feat_drop (see _forward), so no source is masked
+            if any(off for _, off, *_ in srcs):
+                raise SpgnnError("stack: a head-averaged output layer cannot take a gradient at a column offset")
             d_packed[i], d_bias[i], dX[i] = _wide_backward(L, graph, rec, packed[i], [g for g, *_ in srcs],
                                                            tape.training, need_bias[i])
             continue
@@ -607,12 +605,9 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
         for t, off in zip(L.inputs, L.in_offs):
             if t in plan.producer:
                 k_need = off + plan.widths[t]
-        if FOLD_MASK:
-            dX[i] = planes_linear_bwd_input(dY, packed[i], k_need, drop_p=tape.pdrop[i], seed=tape.fseed[i],
-                                            concat_chunks=(L.k_in + 3) // 4) if k_need else None
-            masked.add(i)
-        else:
-            dX[i] = planes_linear_bwd_input(dY, packed[i], k_need) if k_need else None
+        dX[i] = planes_linear_bwd_input(dY, packed[i], k_need, drop_p=tape.pdrop[i], seed=tape.fseed[i],
+                                        concat_chunks=(L.k_in + 3) // 4) if k_need else None
+        masked.add(i)
         del dY, Y, att, ins
     return d_packed, d_bias, d_hw, d_hb
 

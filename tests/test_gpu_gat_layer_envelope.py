@@ -15,11 +15,7 @@ References are plain fp64 formulas on the CPU.  Every output buffer starts as Na
 fails the comparison."""
 import copy
 import ctypes
-import json
-import os
 import re
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -30,7 +26,6 @@ from test_gpu_parity import GRAD_TOL, TRAIN_GRAD_TOL, _random_tree_adj
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NONE, ELU, TANH, RELU, LEAKY = 0, 1, 2, 3, 4         # SPGNN_ACT_*
 LEAKY_SLOPE = 0.01         # F.leaky_relu's default negative_slope: what GATConv(activation=F.leaky_relu) computes
 NEG_SLOPE = 0.2            # LeakyReLU slope of the attention logits
@@ -41,17 +36,13 @@ TOL = 3e-5
 NAN = float("nan")
 
 
-def _load_mods():
+@pytest.fixture(scope="module")
+def mods():
     from oracle import dgl_ops
     from spgnn_b200 import graph as sg, nn as snn, ops, stack
     from spgnn_b200._lib import SpgnnError, lib, ptr, stream
     return dict(dgl_ops=dgl_ops, sg=sg, snn=snn, ops=ops, stack=stack, SpgnnError=SpgnnError, lib=lib, ptr=ptr,
                 stream=stream)
-
-
-@pytest.fixture(scope="module")
-def mods():
-    return _load_mods()
 
 
 def _sms():
@@ -74,25 +65,17 @@ def bwd_smem_bytes(nmax, H, HF, nstages, nwarps):
             + 128)
 
 
-def fwd_shape(n, variant=0):
-    """(threads, rounds per slice); SPGNN_TREE_FWD=1 selects variant 1"""
-    if variant == 1:
-        return (896, 3) if n <= 3 * 112 else (896, 4)
+def fwd_shape(n):
+    """(threads, rounds per slice)"""
     return (512, 5) if n <= 5 * 64 else (512, 6)
 
 
-def bwd_shape(n, variant=3):
-    """(threads, rounds per slice, prefetch depth); SPGNN_TREE_BWD = 0 / 1 / 9 select the alternatives"""
-    if variant == 0:
-        return (512, 5, 5) if n <= 5 * 64 else (512, 6, 6)
-    if variant == 1:
-        return (896, 3, 2) if n <= 3 * 112 else (896, 4, 2)
-    if variant == 9:
-        return (640, 4, 2) if n <= 4 * 80 else (640, 5, 2)
+def bwd_shape(n):
+    """(threads, rounds per slice, prefetch depth)"""
     return (640, 4, 3) if n <= 4 * 80 else (640, 5, 2)
 
 
-def tree_plan(H, F, mean, max_nodes, max_degree, B, n_g, tree, sms, fvar=0, bvar=3):
+def tree_plan(H, F, mean, max_nodes, max_degree, B, n_g, tree, sms):
     """(forward launch or None, backward launch or None) of the per-tree kernels; None: the chunk kernels run."""
     fwd = bwd = None
     if not (tree and B > 0 and 0 < max_nodes <= TREE_MAX_NODES and 0 < max_degree <= 4 and not mean and F % 64 == 0
@@ -100,12 +83,12 @@ def tree_plan(H, F, mean, max_nodes, max_degree, B, n_g, tree, sms, fvar=0, bvar
         return fwd, bwd
     nmax = -(-max_nodes // 32) * 32
     nslices = H * F // 32
-    T, K = fwd_shape(max_nodes, fvar)
+    T, K = fwd_shape(max_nodes)
     st = 2 if fwd_smem_bytes(nmax, H, 2) <= SMEM_LIMIT else 1
     if fwd_smem_bytes(nmax, H, st) <= SMEM_LIMIT:
         fwd = dict(threads=T, kper=K, stages=st, split=min(sms // B, nslices) if B < sms else 1, nslices=nslices)
     if 1 <= n_g <= 2:
-        T, K, PF = bwd_shape(max_nodes, bvar)
+        T, K, PF = bwd_shape(max_nodes)
         st = 2 if bwd_smem_bytes(nmax, H, H * F, 2, T // 32) <= SMEM_LIMIT else 1
         if bwd_smem_bytes(nmax, H, H * F, st, T // 32) <= SMEM_LIMIT:
             bwd = dict(threads=T, kper=K, pf=PF, stages=st, split=H if H > 1 and B * H <= sms else 1,
@@ -260,9 +243,8 @@ def _random_y(N, H, F, res_mode, seed):
 
 
 # ------------------------------------------------------------------------------------------------ spgnn_gat_layer
-def run_layer_case(mods, c, fvar=0, bvar=3):
-    """One forward + backward of spgnn_gat_layer on case ``c`` under the profiler, checked against fp64.  Returns the
-    short names of the kernels that ran."""
+def run_layer_case(mods, c):
+    """One forward + backward of spgnn_gat_layer on case ``c`` under the profiler, checked against fp64."""
     sg, stack, ops, lib, ptr, stream = (mods[k] for k in ("sg", "stack", "ops", "lib", "ptr", "stream"))
     sms = _sms()
     H, F, res, act, mean = c["H"], c["F"], c.get("res", 1), c.get("act", ELU), c.get("mean", False)
@@ -278,10 +260,10 @@ def run_layer_case(mods, c, fvar=0, bvar=3):
     assert N % 32 and g.max_nodes and int(g.batch_num_nodes()[-1]) % 32, "the last tree's boxes must run past N"
 
     # the regime the case claims, from the restated shared-memory arithmetic
-    fwd, bwd = tree_plan(H, F, mean, g.max_nodes, max_degree, g.batch_size, len(gsrc), tree, sms, fvar, bvar)
+    fwd, bwd = tree_plan(H, F, mean, g.max_nodes, max_degree, g.batch_size, len(gsrc), tree, sms)
     claim_f, claim_b = c["regime"]
     assert (fwd is None) == (claim_f == "chunk"), (fwd, claim_f)
-    if claim_f != "chunk" and claim_f != "tree":
+    if claim_f != "chunk":
         assert claim_f == f"tree{fwd['kper']}", (fwd, claim_f)
     assert (bwd is None) == (claim_b == "chunk"), (bwd, claim_b)
     if bwd is not None:
@@ -400,7 +382,6 @@ def run_layer_case(mods, c, fvar=0, bvar=3):
     assert rel_err(dYf[:, er_off:er_off + H], ref["der"]) < TOL, "d er"
     if db is not None:
         assert rel_err(db.cpu(), ref["db"]) < TOL, "dbias"
-    return names
 
 
 def _case(name, H, F, sizes, regime, **kw):
@@ -464,42 +445,6 @@ def test_gat_layer_against_fp64(mods, c):
     d er] and dbias against fp64, after checking the case is in the regime it claims and that exactly the launches of
     that regime ran."""
     run_layer_case(mods, c)
-
-
-_VARIANT_SCRIPT = r"""
-import json, sys
-sys.path[:0] = [sys.argv[1], sys.argv[1] + "/tests"]
-import test_gpu_gat_layer_envelope as t
-m = t._load_mods()
-names = [sorted(t.run_layer_case(m, c, fvar=int(sys.argv[2]), bvar=int(sys.argv[3]))) for c in t.VARIANT_CASES]
-print("KERNELS " + json.dumps(names))
-"""
-
-VARIANT_CASES = [
-    dict(H=2, F=128, sizes=[301, 120], regime=("tree", "tree2"), act=ELU, gsrc=(0.1, 0.0), attn_p=0.1),
-    dict(H=2, F=64, sizes=[384, 33], regime=("tree", "tree2"), act=TANH, sinks=(0.1,)),
-]
-
-
-@pytest.mark.parametrize("fwd_env,bwd_env", [("1", "1"), (None, "0"), (None, "9")])
-def test_alternate_tree_launch_shapes_against_fp64(fwd_env, bwd_env):
-    """SPGNN_TREE_FWD / SPGNN_TREE_BWD are read once per process, hence a subprocess per setting.  Two shapes, one with
-    max_nodes <= 320 and one above, must match fp64 and run the 512- / 896-thread instantiations."""
-    env = dict(os.environ, SPGNN_TREE_BWD=bwd_env)
-    env.pop("SPGNN_TREE_FWD", None)
-    if fwd_env:
-        env["SPGNN_TREE_FWD"] = fwd_env
-    fvar, bvar = int(fwd_env or 0), int(bwd_env)
-    r = subprocess.run([sys.executable, "-c", _VARIANT_SCRIPT, ROOT, str(fvar), str(bvar)], env=env,
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    line = [ln for ln in r.stdout.splitlines() if ln.startswith("KERNELS ")][-1]
-    names = json.loads(line[len("KERNELS "):])
-    threads = {"0": 512, "1": 896, "9": 640}[bwd_env]
-    for case_names in names:
-        assert any(n.startswith("gat_tree_bwd_kernel<") and f",{threads}," in n for n in case_names), case_names
-        ft = 896 if fwd_env == "1" else 512
-        assert any(n.startswith("gat_tree_fwd_kernel<") and f",{ft}," in n for n in case_names), case_names
 
 
 # ------------------------------------------------------------------------------------------------ spgnn_gat_agg (gat.cu)

@@ -1,13 +1,10 @@
 """The aggregate-first output layer (spgnn_gat_aggx_fwd / _bwd + spgnn_wide_linear) over everything its entry points
 accept, not just the H = 2, F = 1024, k_in in {128, 192} of the shipped presets: H in {1, 2, 4}, F % 32 == 0 up to
 H*F = 8192 (ragged last n-tile), k_in < kp (padding inside every 64-column block of XA), a ragged second source,
-activation NONE / ELU / the generic branch, 1..3 gradient sources, either output alone, no bias, and the opt-in CTA-pair
-kernel.  References are fp64 on the CPU: the wide GEMM against its formula, aggx_fwd against an fp64 edge softmax, and
-whole nets against the fp64 oracle with the device's kinks replayed."""
+activation NONE / ELU / the generic branch, 1..3 gradient sources, either output alone and no bias.  References are
+fp64 on the CPU: the wide GEMM against its formula, aggx_fwd against an fp64 edge softmax, and whole nets against the
+fp64 oracle with the device's kinks replayed."""
 import ctypes
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -19,7 +16,6 @@ from test_gpu_parity import (GRAD_TOL, NET_CLS, TOL, TRAIN_GRAD_TOL, _device_bat
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SMS = 148
 ACT_NONE, ACT_ELU, ACT_TANH = 0, 1, 2          # tanh takes the generic wide_act<-1> branch of the epilogue
 GEMM_TOL = 4e-5                                # split-bf16 planes GEMMs vs fp64 (test_linear_fwd_bwd_against_fp64)
@@ -327,55 +323,3 @@ def test_aggregate_first_nets_outside_the_shipped_widths_vs_oracle(mods, name, t
         err = float((wide_grads[k].double() - p.grad.double()).abs().max())
         assert err <= 5e-5 * float(p.grad.abs().max()) or err <= 1e-6 * gmax, (name, k, err)
 
-
-# ------------------------------------------------------------------------------------------------ CTA pairs
-_PAIR_SCRIPT = r"""
-import sys, torch
-sys.path[:0] = [sys.argv[1], sys.argv[1] + "/tests"]
-from spgnn_b200 import stack
-from test_gpu_output_layer_envelope import run_wide, wide_operands
-H, F, k_in, has_res, act, M = (int(v) for v in sys.argv[2:8])
-XA, kp, W, b = wide_operands(stack, M, H, F, k_in, has_res, seed=M + H * F)
-g = torch.randn(M, F, generator=torch.Generator().manual_seed(M)).cuda()
-with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
-    out, P = run_wide(stack, XA, kp, k_in, M, H, F, has_res, W, b, act, 0)
-    dpre, db = run_wide(stack, XA, kp, k_in, M, H, F, has_res, W, b, act, 1, grads=[g])
-    torch.cuda.synchronize()
-kernels = sorted({e.name for e in prof.events() if "wide" in e.name})
-torch.save(dict(out=out.cpu(), P=P.float().cpu(), dpre=dpre.float().cpu(), db=db.cpu(), kernels=kernels), sys.argv[8])
-"""
-
-
-@pytest.mark.parametrize("H,F,k_in,has_res,act,M", [(2, 1024, 192, 1, ACT_ELU, 40001), (4, 512, 100, 0, ACT_TANH, 38913),
-                                                    (1, 256, 64, 1, ACT_NONE, 39041)])
-def test_cta_pair_wide_kernel_against_fp64_and_the_single_cta_kernel(mods, H, F, k_in, has_res, act, M, tmp_path):
-    """SPGNN_WIDE_PAIR=1 (read once per process, hence the subprocess) on shapes where the pair kernel is eligible:
-    F % BN == 0 and at least 4 m-tiles per co-resident cluster (~74 on 148 SMs).  Modes 0 and 1 against fp64 and
-    against the single-CTA kernel of this process."""
-    stack = mods["stack"]
-    BN = min(256 // H, F)
-    assert F % BN == 0 and -(-M // 128) >= 4 * (SMS // 2)
-    res = {}
-    for pair in ("1", "0"):
-        path = tmp_path / f"pair{pair}.pt"
-        env = dict(os.environ, SPGNN_WIDE_PAIR=pair)
-        r = subprocess.run([sys.executable, "-c", _PAIR_SCRIPT, ROOT, str(H), str(F), str(k_in), str(has_res), str(act),
-                            str(M), str(path)], env=env, capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stderr[-3000:]
-        res[pair] = torch.load(path, weights_only=False)
-    assert any("wide_pair_kernel" in k for k in res["1"]["kernels"]), res["1"]["kernels"]
-    assert not any("wide_pair_kernel" in k for k in res["0"]["kernels"]), res["0"]["kernels"]
-    assert any("wide_kernel" in k for k in res["0"]["kernels"]), res["0"]["kernels"]
-    XA, kp, W, b = wide_operands(stack, M, H, F, k_in, has_res, seed=M + H * F)
-    pre = wide_pre64(XA, kp, W, b, M, H, F, k_in, has_res)
-    del XA
-    ref = _act64(pre, act).mean(0)
-    g = torch.randn(M, F, generator=torch.Generator().manual_seed(M)).double()
-    dref = torch.cat([g / H * _act_grad64(pre[h], act) for h in range(H)], 1)
-    for pair, r in res.items():
-        assert rel_err(r["out"], ref) < GEMM_TOL, pair
-        assert rel_err(r["P"], ref) < GEMM_TOL, pair
-        assert rel_err(r["dpre"], dref) < GEMM_TOL, pair
-        assert rel_err(r["db"], dref.sum(0)) < GEMM_TOL, pair
-    for k in ("out", "P", "dpre"):
-        assert rel_err(res["1"][k], res["0"][k].double()) < 1e-5, k
