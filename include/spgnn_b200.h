@@ -342,6 +342,22 @@ int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp
                       const float* g0, int64_t ldg0, const float* g1, int64_t ldg1, const float* g2, int64_t ldg2,
                       uint16_t* dpre, int64_t ldd, int64_t psd, float* dbias,
                       void* ws, int64_t ws_bytes, void* stream);
+/* Mode 0 that also writes dact fp32 [N, ldda >= H*F] <- act'(pre_h) for every head h (column h*F + f), the values
+ * mode 1 recomputes, bit for bit.  Same ws as spgnn_wide_linear. */
+int spgnn_wide_linear_fwd_dact(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp, int64_t k_in, int64_t M,
+                               int H, int F, int has_res, const float* W, int64_t ldw, const float* bias, int act,
+                               float* out, int64_t ldo, uint16_t* out_planes, int64_t ldp, int64_t psp,
+                               float* dact, int64_t ldda, void* ws, int64_t ws_bytes, void* stream);
+/* The dpre of mode 1 when the layer output feeds a linear head (W_head [C, ldwh >= F], C <= 64) and dact was saved:
+ * gl = the head's output-gradient planes [M, C] (ld ldgl, plane stride psgl);  with g = gl * W_head (the head's dX,
+ * never stored) and up to two further fp32 [M, F] sources g0, g1,
+ *   dpre planes [M, H*F] <- (g0 + g1 + g) / H * dact_h;  dbias [H*F] (optional) <- column sums of dpre.
+ * ws: spgnn_wide_dpre_ws bytes. */
+int64_t spgnn_wide_dpre_ws(int64_t H, int64_t F);
+int spgnn_wide_dpre(const uint16_t* gl, int64_t ldgl, int64_t psgl, int64_t C, int64_t M, int H, int F,
+                    const float* W_head, int64_t ldwh, const float* dact, int64_t ldda,
+                    const float* g0, int64_t ldg0, const float* g1, int64_t ldg1,
+                    uint16_t* dpre, int64_t ldd, int64_t psd, float* dbias, void* ws, int64_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Weighted-sum aggregation (DGL SpMM copy_u.sum with degree norms): GraphConv, GINConv-mean, SAGEConv mean / gcn.

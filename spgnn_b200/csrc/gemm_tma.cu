@@ -415,17 +415,23 @@ __global__ void __launch_bounds__(kThreads, 1) nt_pair_kernel(const __grid_const
 // A = XA planes [M, (H+1)*kp] (block h = Ax_h, block H = x), B = weight planes [H*F, nparts*kp].  A tile is 128 rows x
 // BN columns x H heads: H accumulators of BN TMEM columns each (x 2 buffers), the k-loop runs head after head; the
 // epilogue walks the heads one at a time, so per thread only the running mean (mode 0) or the incoming gradient
-// (mode 1) stays in registers.
+// (mode 1) stays in registers.  Mode 0 can also write act'(pre_h) of every head (dact), which mode 2 reads back.
+// Mode 2 (dpre from the gradient of a linear head on the output): A = the head's output-gradient planes [M, C],
+// B = W_head^T planes [F, 64]; ONE accumulator (the head's dX, the same for every head h), and the epilogue forms
+// dpre_h = (sum of the fp32 sources + acc) / H * dact_h -- the operation order of mode 1 with the head's dX as its
+// last source, without recomputing the forward GEMM.
 struct WideMaps { CUtensorMap a, b; };
 struct WideArgs {
     int mode, H, F, act;
     const float* bias;
     float* out; int64_t ldo;
     __nv_bfloat16* outp; int64_t ldp, psp;
+    float* dact; int64_t ldda;                 // mode 0: written when non-null; mode 2: read
     const float* g[3]; int64_t ldg[3]; int n_g;
     __nv_bfloat16* dpre; int64_t ldd, psd;
     float* dbias_ws;
     int64_t M; int BN, nt_n; int64_t nt_m;
+    int hacc;                                  // accumulators per tile: H (modes 0 and 1) or 1 (mode 2)
     int kbp, nparts, kp;
     int stages, stage_bytes;
 };
@@ -453,6 +459,18 @@ __device__ __forceinline__ float wide_act_grad_pre(float x, int act) {
     if (ACT == SPGNN_ACT_NONE) return 1.f;
     return act_grad_from_out(act_fwd(x, act, kGatLeakySlope), act, kGatLeakySlope);
 }
+// run += act(x) and d = act'(x): the values of wide_act and wide_act_grad_pre, bit for bit
+template <int ACT>
+__device__ __forceinline__ void wide_act_and_grad(float x, int act, float& run, float& d) {
+    if (ACT == SPGNN_ACT_ELU) {
+        const float e = exp_fast(x);
+        run += x > 0.f ? x : e - 1.f;
+        d = x > 0.f ? 1.f : e;
+    } else {
+        run += wide_act<ACT>(x, act);
+        d = wide_act_grad_pre<ACT>(x, act);
+    }
+}
 __device__ __forceinline__ void st_planes4(__nv_bfloat16* q, int64_t ps, float4 d) {
     uint32_t h0, l0, h1, l1;
     split2(d.x, d.y, h0, l0);
@@ -466,7 +484,8 @@ __device__ __forceinline__ void st_planes4(__nv_bfloat16* q, int64_t ps, float4 
 // hides behind the MMAs of this tile.  The MMA work per output element is small here (K = 2 x 192), so the tile is
 // only hidden behind the tensor pipe if the epilogue stays near ~1 issue slot per element: MODE and ACT are template
 // parameters, the staging tile is addressed in the shared window, row pointers are hoisted out of the head loop.
-template <int ACT, int MODE>
+// DACT (mode 0): also store act'(pre_h) of every head into dact [M, H*F].
+template <int ACT, int MODE, bool DACT>
 __device__ __forceinline__ void wide_epilogue_tile(const WideArgs& g, uint32_t stg, float* dbias_row, uint32_t taddr,
                                                    int64_t m0, int n0, int ncols, int warp, int lane,
                                                    uint32_t full_bar, uint32_t full_par) {
@@ -531,6 +550,8 @@ __device__ __forceinline__ void wide_epilogue_tile(const WideArgs& g, uint32_t s
             const int col = colq + c0;
             __nv_bfloat16* dp = MODE == 1 ? g.dpre + row0 * g.ldd + col : nullptr;
             const int64_t dstep = 8 * g.ldd;
+            float* da = DACT ? g.dact + row0 * g.ldda + col : nullptr;
+            const int64_t astep = 8 * g.ldda;
             uint32_t v[16];
             tmem_ld16(taddr + c0, v);
             for (int h = 0; h < g.H; ++h) {
@@ -545,7 +566,14 @@ __device__ __forceinline__ void wide_epilogue_tile(const WideArgs& g, uint32_t s
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
                     float4 x = ld_shared4(st_r[i]);
-                    if (MODE == 0) {
+                    if (MODE == 0 && DACT) {
+                        float4 a;
+                        wide_act_and_grad<ACT>(x.x + bv.x, g.act, run[q][i].x, a.x);
+                        wide_act_and_grad<ACT>(x.y + bv.y, g.act, run[q][i].y, a.y);
+                        wide_act_and_grad<ACT>(x.z + bv.z, g.act, run[q][i].z, a.z);
+                        wide_act_and_grad<ACT>(x.w + bv.w, g.act, run[q][i].w, a.w);
+                        if (i < nrow) st4(da + i * astep + h * g.F, a);
+                    } else if (MODE == 0) {
                         run[q][i].x += wide_act<ACT>(x.x + bv.x, g.act);
                         run[q][i].y += wide_act<ACT>(x.y + bv.y, g.act);
                         run[q][i].z += wide_act<ACT>(x.z + bv.z, g.act);
@@ -591,6 +619,122 @@ __device__ __forceinline__ void wide_epilogue_tile(const WideArgs& g, uint32_t s
     }
 }
 
+// Mode 2 epilogue of one 128 x BN tile for one warp (same thread layout as wide_epilogue_tile).  The accumulator is
+// the head's dX g (one per tile); run = (sources... + g) / H is formed once, then every head streams its dact in and
+// its dpre planes out (the tile is bound by that traffic).
+__device__ __forceinline__ void wide_dpre_tile(const WideArgs& g, uint32_t stg, float* dbias_row, uint32_t taddr,
+                                               int64_t m0, int n0, int ncols, int warp, int lane, uint32_t full_bar,
+                                               uint32_t full_par) {
+    const int quad = warp & 3, part = warp >> 2;
+    const int r0 = lane >> 2, cq = lane & 3;
+    const float inv_h = 1.f / (float)g.H;
+    const int64_t row0 = m0 + quad * 32 + r0;
+    const int nrow = (int)max((int64_t)0, min((int64_t)4, (g.M - row0 + 7) / 8));
+    const uint32_t st_w = stg + lane * 64;
+    const int sw_w = (lane >> 1) & 3;
+    uint32_t st_r[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int r = r0 + 8 * i;
+        st_r[i] = stg + r * 64 + ((cq ^ ((r >> 1) & 3)) << 4);
+    }
+    const int colq = n0 + cq * 4;
+    const int64_t dstep = 8 * g.ldd, astep = 8 * g.ldda;
+    for (int cg = 0; cg < ncols; cg += 128) {
+        float4 run[2][4];
+        // the fp32 sources first (their loads overlap the MMAs), in the order mode 1 sums them
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const int c0 = cg + q * 64 + part * 16;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                run[q][i] = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (g.n_g > 0 && i < nrow && c0 < ncols)
+                    run[q][i] = ldg4(g.g[0] + (row0 + 8 * i) * g.ldg[0] + colq + c0);
+            }
+        }
+        for (int s = 1; s < g.n_g; ++s) {
+#pragma unroll
+            for (int q = 0; q < 2; ++q) {
+                const int c0 = cg + q * 64 + part * 16;
+                float4 t[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                    t[i] = (i < nrow && c0 < ncols) ? ldg4(g.g[s] + (row0 + 8 * i) * g.ldg[s] + colq + c0)
+                                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    run[q][i].x += t[i].x; run[q][i].y += t[i].y; run[q][i].z += t[i].z; run[q][i].w += t[i].w;
+                }
+            }
+        }
+        if (cg == 0) {
+            mbar_wait(full_bar, full_par);
+            tc_fence_after();
+        }
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const int c0 = cg + q * 64 + part * 16;
+            if (c0 >= ncols) break;
+            uint32_t v[16];
+            tmem_ld16(taddr + c0, v);
+            tmem_ld_wait();
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+                st_shared4(st_w + ((j ^ sw_w) << 4), v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+            __syncwarp();
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const float4 x = ld_shared4(st_r[i]);
+                float4& r = run[q][i];
+                if (g.n_g > 0) { r.x += x.x; r.y += x.y; r.z += x.z; r.w += x.w; }
+                else r = x;
+                r.x *= inv_h; r.y *= inv_h; r.z *= inv_h; r.w *= inv_h;
+            }
+            __syncwarp();
+        }
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const int c0 = cg + q * 64 + part * 16;
+            if (c0 >= ncols) break;
+            const int col = colq + c0;
+            const float* pa = g.dact + row0 * g.ldda + col;
+            __nv_bfloat16* dp = g.dpre + row0 * g.ldd + col;
+            for (int h = 0; h < g.H; ++h) {
+                float4 a[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                    a[i] = i < nrow ? ldg4(pa + i * astep + h * g.F) : make_float4(0.f, 0.f, 0.f, 0.f);
+                float4 bs = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    if (i < nrow) {
+                        float4 d;
+                        d.x = run[q][i].x * a[i].x;
+                        d.y = run[q][i].y * a[i].y;
+                        d.z = run[q][i].z * a[i].z;
+                        d.w = run[q][i].w * a[i].w;
+                        st_planes4(dp + i * dstep + h * g.F, g.psd, d);
+                        bs.x += d.x; bs.y += d.y; bs.z += d.z; bs.w += d.w;
+                    }
+                }
+                if (dbias_row) {
+#pragma unroll
+                    for (int o = 4; o < 32; o <<= 1) {
+                        bs.x += __shfl_xor_sync(kFull, bs.x, o); bs.y += __shfl_xor_sync(kFull, bs.y, o);
+                        bs.z += __shfl_xor_sync(kFull, bs.z, o); bs.w += __shfl_xor_sync(kFull, bs.w, o);
+                    }
+                    if (lane < 4) {
+                        float* p = dbias_row + h * g.F + col;
+                        atomicAdd(p, bs.x); atomicAdd(p + 1, bs.y); atomicAdd(p + 2, bs.z); atomicAdd(p + 3, bs.w);
+                    }
+                }
+            }
+        }
+    }
+}
+
+template <int MODE, bool DACT>
 __global__ void __launch_bounds__(kWideThreads, 1) wide_kernel(const __grid_constant__ WideMaps maps, const WideArgs g) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -637,14 +781,14 @@ __global__ void __launch_bounds__(kWideThreads, 1) wide_kernel(const __grid_cons
             const int ncols = min(g.BN, g.F - n0);
             const uint32_t taddr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(buf * accw);
             const uint32_t fb = smem_u32(&sh->tmem_full[buf]);
-            if (g.mode == 0) {
-                if (g.act == SPGNN_ACT_ELU) wide_epilogue_tile<SPGNN_ACT_ELU, 0>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else if (g.act == SPGNN_ACT_NONE) wide_epilogue_tile<SPGNN_ACT_NONE, 0>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else wide_epilogue_tile<-1, 0>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
+            if (MODE == 2) {
+                wide_dpre_tile(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
+            } else if (g.act == SPGNN_ACT_ELU) {
+                wide_epilogue_tile<SPGNN_ACT_ELU, MODE, DACT>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
+            } else if (g.act == SPGNN_ACT_NONE) {
+                wide_epilogue_tile<SPGNN_ACT_NONE, MODE, DACT>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
             } else {
-                if (g.act == SPGNN_ACT_ELU) wide_epilogue_tile<SPGNN_ACT_ELU, 1>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else if (g.act == SPGNN_ACT_NONE) wide_epilogue_tile<SPGNN_ACT_NONE, 1>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
-                else wide_epilogue_tile<-1, 1>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
+                wide_epilogue_tile<-1, MODE, DACT>(g, stg, dbias_row, taddr, m0, n0, ncols, warp, lane, fb, par);
             }
             tc_fence_before();
             mbar_arrive(smem_u32(&sh->tmem_empty[buf]));
@@ -663,7 +807,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) wide_kernel(const __grid_cons
                 const uint32_t idesc = make_idesc(ncols, false);
                 mbar_wait(smem_u32(&sh->tmem_empty[buf]), par ^ 1);
                 tc_fence_after();
-                for (int h = 0; h < g.H; ++h) {
+                for (int h = 0; h < g.hacc; ++h) {
                     const uint32_t tmem_d = tbase + (uint32_t)(buf * accw + h * g.BN);
                     for (int kb = 0; kb < nkb; ++kb, ++kcount) {
                         const int s = kcount % g.stages;
@@ -700,7 +844,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) wide_kernel(const __grid_cons
         for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             const int m0 = (int)((tile / g.nt_n) * BM);
             const int n0 = (int)(tile % g.nt_n) * g.BN;
-            for (int h = 0; h < g.H; ++h) {
+            for (int h = 0; h < g.hacc; ++h) {
                 for (int kb = 0; kb < nkb; ++kb, ++kcount) {
                     const int s = kcount % g.stages;
                     const uint32_t sp = (kcount / g.stages) & 1;
@@ -1204,12 +1348,58 @@ extern "C" int64_t spgnn_wide_linear_ws(int64_t H, int64_t F, int64_t kp, int ha
     return b + 256 + (int64_t)sm_count() * H * F * (int64_t)sizeof(float) + 256;
 }
 
-extern "C" int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp, int64_t k_in, int64_t M,
-                                 int H, int F, int has_res, const float* W, int64_t ldw, const float* bias, int act,
-                                 int mode, float* out, int64_t ldo, uint16_t* out_planes, int64_t ldp, int64_t psp,
-                                 const float* g0, int64_t ldg0, const float* g1, int64_t ldg1, const float* g2,
-                                 int64_t ldg2, uint16_t* dpre, int64_t ldd, int64_t psd, float* dbias, void* ws,
-                                 int64_t ws_bytes, void* stream) {
+namespace {
+// Tiling of the wide GEMM: 128 x BN tiles, BN = 256 / H columns per head (H accumulators fill the 512 TMEM columns
+// of two buffers), as many pipeline stages as fit.
+int wide_tiling(WideArgs& a) {
+    a.BN = 256 / a.H;
+    if (a.BN > a.F) a.BN = a.F;
+    a.nt_n = (int)ceil_div(a.F, a.BN);
+    a.nt_m = ceil_div(a.M, BM);
+    a.stage_bytes = kABytes + a.BN * 256;
+    a.stages = (kSmemLimit - kWideFixed) / a.stage_bytes;
+    if (a.stages > kMaxStages) a.stages = kMaxStages;
+    SPGNN_REQUIRE(a.stages >= 2, "wide_linear: not enough shared memory for two pipeline stages");
+    return SPGNN_OK;
+}
+
+// Launches the kernel of a.mode with maps and tiling set up; dbias (modes 1 and 2, optional) goes through per-CTA
+// partial rows at part_ws, reduced in fixed order.
+int wide_launch(const WideMaps& maps, WideArgs& a, float* dbias, void* part_ws, cudaStream_t st) {
+    static DeviceOnce attr;
+    if (attr.pending()) {
+        SPGNN_CUDA_OK(cudaFuncSetAttribute(wide_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+        SPGNN_CUDA_OK(cudaFuncSetAttribute(wide_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+        SPGNN_CUDA_OK(cudaFuncSetAttribute(wide_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+        SPGNN_CUDA_OK(cudaFuncSetAttribute(wide_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+        attr.done();
+    }
+    const int64_t HF = (int64_t)a.H * a.F;
+    const int64_t tiles = a.nt_m * a.nt_n;
+    const unsigned grid = (unsigned)(tiles < sm_count() ? tiles : sm_count());
+    float* part = nullptr;
+    if (a.mode != 0 && dbias) {
+        part = reinterpret_cast<float*>(((uintptr_t)part_ws + 255) & ~(uintptr_t)255);
+        a.dbias_ws = part;
+        SPGNN_CUDA_OK(cudaMemsetAsync(part, 0, (size_t)grid * HF * sizeof(float), st));
+    }
+    if (a.mode == 0 && a.dact) wide_kernel<0, true><<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
+    else if (a.mode == 0) wide_kernel<0, false><<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
+    else if (a.mode == 1) wide_kernel<1, false><<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
+    else wide_kernel<2, false><<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
+    SPGNN_LAUNCH_OK();
+    if (part) {
+        wide_dbias_reduce_kernel<<<(unsigned)ceil_div(HF, 128), 128, 0, st>>>(part, grid, HF, dbias);
+        SPGNN_LAUNCH_OK();
+    }
+    return SPGNN_OK;
+}
+
+int wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp, int64_t k_in, int64_t M, int H, int F,
+                int has_res, const float* W, int64_t ldw, const float* bias, int act, int mode, float* out, int64_t ldo,
+                uint16_t* out_planes, int64_t ldp, int64_t psp, float* dact, int64_t ldda, const float* g0,
+                int64_t ldg0, const float* g1, int64_t ldg1, const float* g2, int64_t ldg2, uint16_t* dpre,
+                int64_t ldd, int64_t psd, float* dbias, void* ws, int64_t ws_bytes, void* stream) {
     SPGNN_REQUIRE(XA && W && ws && M > 0 && k_in > 0, "wide_linear: bad argument");
     SPGNN_REQUIRE(H == 1 || H == 2 || H == 4, "wide_linear: H must be 1, 2 or 4 (got %d)", H);
     SPGNN_REQUIRE(F > 0 && F % 32 == 0 && (int64_t)H * F <= 8192, "wide_linear: F (%d) must be a multiple of 32, H*F <= 8192", F);
@@ -1220,13 +1410,16 @@ extern "C" int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa,
     SPGNN_REQUIRE(M < (1ll << 31), "wide_linear: too many rows");
     WideMaps maps;
     WideArgs a{};
-    a.mode = mode; a.H = H; a.F = F; a.act = act; a.bias = bias; a.M = M;
+    a.mode = mode; a.H = H; a.F = F; a.act = act; a.bias = bias; a.M = M; a.hacc = H;
     if (mode == 0) {
         SPGNN_REQUIRE(out || out_planes, "wide_linear: no output");
         SPGNN_REQUIRE(!out || (ldo % 4 == 0 && ldo >= F && ((uintptr_t)out & 15) == 0), "wide_linear: out alignment");
         SPGNN_REQUIRE(!out_planes || (ldp % 4 == 0 && ldp >= F && psp % 4 == 0 && ((uintptr_t)out_planes & 7) == 0),
                       "wide_linear: out planes alignment");
+        SPGNN_REQUIRE(!dact || (ldda % 4 == 0 && ldda >= (int64_t)H * F && ((uintptr_t)dact & 15) == 0),
+                      "wide_linear: dact must be 16-byte aligned with ld %% 4 == 0 and ld >= H*F");
         a.out = out; a.ldo = ldo; a.outp = reinterpret_cast<__nv_bfloat16*>(out_planes); a.ldp = ldp; a.psp = psp;
+        a.dact = dact; a.ldda = ldda;
     } else {
         SPGNN_REQUIRE(g0 && dpre, "wide_linear: mode 1 needs a gradient source and the dpre planes");
         SPGNN_REQUIRE(ldd % 4 == 0 && ldd >= (int64_t)H * F && psd % 4 == 0 && ((uintptr_t)dpre & 7) == 0,
@@ -1242,11 +1435,6 @@ extern "C" int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa,
         a.dpre = reinterpret_cast<__nv_bfloat16*>(dpre); a.ldd = ldd; a.psd = psd;
     }
     cudaStream_t st = as_stream(stream);
-    static DeviceOnce attr;
-    if (attr.pending()) {
-        SPGNN_CUDA_OK(cudaFuncSetAttribute(wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
-        attr.done();
-    }
     const int nparts = has_res ? 2 : 1;
     const int64_t HF = (int64_t)H * F, ldb = nparts * kp;
     __nv_bfloat16* hi = reinterpret_cast<__nv_bfloat16*>(((uintptr_t)ws + 127) & ~(uintptr_t)127);
@@ -1256,35 +1444,85 @@ extern "C" int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa,
                                                                  hi + HF * ldb + p * kp, ldb);
         SPGNN_LAUNCH_OK();
     }
-    a.BN = 256 / H;
-    if (a.BN > F) a.BN = F;
-    a.nt_n = (int)ceil_div(F, a.BN);
-    a.nt_m = ceil_div(M, BM);
+    int rc = wide_tiling(a);
+    if (rc) return rc;
     a.kbp = (int)(kp / BK); a.nparts = nparts; a.kp = (int)kp;
-    int rc = make_planes_map(&maps.a, XA, M, (int64_t)(H + 1) * kp, ldxa, psxa, BK, BM);
+    rc = make_planes_map(&maps.a, XA, M, (int64_t)(H + 1) * kp, ldxa, psxa, BK, BM);
     if (rc) return rc;
     rc = make_planes_map(&maps.b, hi, HF, ldb, ldb, HF * ldb, BK, a.BN);
     if (rc) return rc;
     // A CTA-pair variant was slower at the bench size and was removed (profiles/r02_wide_pair_probe.txt).
-    a.stage_bytes = kABytes + a.BN * 256;
-    a.stages = (kSmemLimit - kWideFixed) / a.stage_bytes;
-    if (a.stages > kMaxStages) a.stages = kMaxStages;
-    SPGNN_REQUIRE(a.stages >= 2, "wide_linear: not enough shared memory for two pipeline stages");
-    const int64_t tiles = a.nt_m * a.nt_n;
-    const unsigned grid = (unsigned)(tiles < sm_count() ? tiles : sm_count());
-    float* part = nullptr;
-    if (mode == 1 && dbias) {
-        part = reinterpret_cast<float*>(((uintptr_t)(hi + 2 * HF * ldb) + 255) & ~(uintptr_t)255);
-        a.dbias_ws = part;
-        SPGNN_CUDA_OK(cudaMemsetAsync(part, 0, (size_t)grid * HF * sizeof(float), st));
+    return wide_launch(maps, a, dbias, hi + 2 * HF * ldb, st);
+}
+}  // namespace
+
+extern "C" int spgnn_wide_linear(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp, int64_t k_in, int64_t M,
+                                 int H, int F, int has_res, const float* W, int64_t ldw, const float* bias, int act,
+                                 int mode, float* out, int64_t ldo, uint16_t* out_planes, int64_t ldp, int64_t psp,
+                                 const float* g0, int64_t ldg0, const float* g1, int64_t ldg1, const float* g2,
+                                 int64_t ldg2, uint16_t* dpre, int64_t ldd, int64_t psd, float* dbias, void* ws,
+                                 int64_t ws_bytes, void* stream) {
+    return wide_linear(XA, ldxa, psxa, kp, k_in, M, H, F, has_res, W, ldw, bias, act, mode, out, ldo, out_planes, ldp,
+                       psp, nullptr, 0, g0, ldg0, g1, ldg1, g2, ldg2, dpre, ldd, psd, dbias, ws, ws_bytes, stream);
+}
+
+extern "C" int spgnn_wide_linear_fwd_dact(const uint16_t* XA, int64_t ldxa, int64_t psxa, int64_t kp, int64_t k_in,
+                                          int64_t M, int H, int F, int has_res, const float* W, int64_t ldw,
+                                          const float* bias, int act, float* out, int64_t ldo, uint16_t* out_planes,
+                                          int64_t ldp, int64_t psp, float* dact, int64_t ldda, void* ws,
+                                          int64_t ws_bytes, void* stream) {
+    SPGNN_REQUIRE(dact, "wide_linear_fwd_dact: no dact output");
+    return wide_linear(XA, ldxa, psxa, kp, k_in, M, H, F, has_res, W, ldw, bias, act, 0, out, ldo, out_planes, ldp,
+                       psp, dact, ldda, nullptr, 0, nullptr, 0, nullptr, 0, nullptr, 0, 0, nullptr, ws, ws_bytes,
+                       stream);
+}
+
+extern "C" int64_t spgnn_wide_dpre_ws(int64_t H, int64_t F) {
+    const int64_t b = 2 * F * BK * (int64_t)sizeof(__nv_bfloat16);
+    return b + 256 + (int64_t)sm_count() * H * F * (int64_t)sizeof(float) + 256;
+}
+
+extern "C" int spgnn_wide_dpre(const uint16_t* GL, int64_t ldgl, int64_t psgl, int64_t C, int64_t M, int H, int F,
+                               const float* Wh, int64_t ldwh, const float* dact, int64_t ldda, const float* g0,
+                               int64_t ldg0, const float* g1, int64_t ldg1, uint16_t* dpre, int64_t ldd, int64_t psd,
+                               float* dbias, void* ws, int64_t ws_bytes, void* stream) {
+    SPGNN_REQUIRE(GL && Wh && dact && dpre && ws && M > 0, "wide_dpre: bad argument");
+    SPGNN_REQUIRE(C > 0 && C <= BK && ldgl >= C && ldwh >= F, "wide_dpre: the head has 1..64 outputs (got %lld)",
+                  (long long)C);
+    SPGNN_REQUIRE(H == 1 || H == 2 || H == 4, "wide_dpre: H must be 1, 2 or 4 (got %d)", H);
+    SPGNN_REQUIRE(F > 0 && F % 32 == 0 && (int64_t)H * F <= 8192, "wide_dpre: F (%d) must be a multiple of 32, H*F <= 8192", F);
+    SPGNN_REQUIRE(ldda % 4 == 0 && ldda >= (int64_t)H * F && ((uintptr_t)dact & 15) == 0,
+                  "wide_dpre: dact must be 16-byte aligned with ld %% 4 == 0 and ld >= H*F");
+    SPGNN_REQUIRE(ldd % 4 == 0 && ldd >= (int64_t)H * F && psd % 4 == 0 && ((uintptr_t)dpre & 7) == 0,
+                  "wide_dpre: dpre planes alignment");
+    SPGNN_REQUIRE(ws_bytes >= spgnn_wide_dpre_ws(H, F), "wide_dpre: workspace too small");
+    SPGNN_REQUIRE(M < (1ll << 31), "wide_dpre: too many rows");
+    WideMaps maps;
+    WideArgs a{};
+    a.mode = 2; a.H = H; a.F = F; a.act = SPGNN_ACT_NONE; a.M = M; a.hacc = 1;
+    a.dact = const_cast<float*>(dact); a.ldda = ldda;
+    const float* gs[2] = {g0, g1};
+    const int64_t lds[2] = {ldg0, ldg1};
+    for (int s = 0; s < 2; ++s) {
+        if (!gs[s]) continue;
+        SPGNN_REQUIRE(lds[s] % 4 == 0 && lds[s] >= F && ((uintptr_t)gs[s] & 15) == 0,
+                      "wide_dpre: gradient source %d must be 16-byte aligned with ld %% 4 == 0", s);
+        a.g[a.n_g] = gs[s]; a.ldg[a.n_g] = lds[s]; ++a.n_g;
     }
-    wide_kernel<<<grid, kWideThreads, kSmemLimit, st>>>(maps, a);
+    a.dpre = reinterpret_cast<__nv_bfloat16*>(dpre); a.ldd = ldd; a.psd = psd;
+    cudaStream_t st = as_stream(stream);
+    // B = W_head^T [F, C] split into planes with K padded to one 64-wide block, as spgnn_planes_linear_bwd_input does
+    __nv_bfloat16* hi = reinterpret_cast<__nv_bfloat16*>(((uintptr_t)ws + 127) & ~(uintptr_t)127);
+    split_weight_kernel<<<split_grid(F * BK), 256, 0, st>>>(Wh, ldwh, 1, 0, F, BK, 0, 0, 0, (int)C, hi, hi + F * BK, BK);
     SPGNN_LAUNCH_OK();
-    if (part) {
-        wide_dbias_reduce_kernel<<<(unsigned)ceil_div(HF, 128), 128, 0, st>>>(part, grid, HF, dbias);
-        SPGNN_LAUNCH_OK();
-    }
-    return SPGNN_OK;
+    int rc = wide_tiling(a);
+    if (rc) return rc;
+    a.kbp = 1; a.nparts = 1; a.kp = BK;
+    rc = make_planes_map(&maps.a, GL, M, C, ldgl, psgl, BK, BM);
+    if (rc) return rc;
+    rc = make_planes_map(&maps.b, hi, F, BK, BK, F * BK, BK, a.BN);
+    if (rc) return rc;
+    return wide_launch(maps, a, dbias, hi + 2 * F * BK, st);
 }
 
 extern "C" int64_t spgnn_planes_linear_bwd_input_ws(int64_t N, int64_t K) {

@@ -79,6 +79,11 @@ class _Wide(ctypes.Structure):
 # Aggregate-first evaluation of head-averaged output layers (include/spgnn_b200.h, spgnn_gat_wide).  Switch off to
 # run every layer through the projection-first kernels (tests compare the two).
 WIDE_OUTPUT_LAYER = True
+# Training an aggregate-first output layer that feeds the head (train mode, tape kept): the forward keeps act'(pre) of
+# every head and the backward builds the pre-activation gradient from the head's output gradient in one memory-bound
+# pass (spgnn_wide_dpre) instead of the head's dX GEMM plus a recompute of the wide GEMM (spgnn_wide_linear mode 1).
+# Costs H*F*4 bytes per node from the forward to the backward.  Off: mode 1 (tests compare the two).
+WIDE_SAVED_DACT = True
 # One CTA per graph with the graph's rows staged in shared memory (spgnn_gat_layer.node_off).  Off: chunk kernels.
 TREE_KERNELS = True
 
@@ -308,8 +313,9 @@ def _forward(plan: StackPlan, graph, ext, packed, biases, head, training, keep):
         if len(keys) > 2:
             raise SpgnnError("stack: more than two dropout variants of one tensor are not supported")
         if L.wide and WIDE_OUTPUT_LAYER and all(k < 0 for k in keys):
+            save_dact = keep and training and want_head and WIDE_SAVED_DACT and not ops.tracing()
             out32, P, rec = _wide_forward(L, graph, ins, packed[i], biases[i], conv, training, aseed[i], is_out,
-                                          bool(keys))
+                                          bool(keys), save_dact)
             if P is not None:
                 variants[(L.output, -1)] = P
             if is_out:
@@ -382,7 +388,7 @@ def _forward(plan: StackPlan, graph, ext, packed, biases, head, training, keep):
 
 class _WideRec:
     """Tape record of a layer evaluated aggregate-first."""
-    __slots__ = ("XA", "att", "eler", "bias", "aseed", "kp")
+    __slots__ = ("XA", "att", "eler", "bias", "aseed", "kp", "dact")
 
 
 def _wide_desc(L, graph, conv, training, aseed, XA, kp, eler, att):
@@ -399,8 +405,9 @@ def _wide_desc(L, graph, conv, training, aseed, XA, kp, eler, att):
     return d
 
 
-def _wide_forward(L, graph, ins, W, bias, conv, training, aseed, want_out, want_planes):
-    """Head-averaged output layer, aggregate-first (spgnn_gat_aggx_fwd + spgnn_wide_linear mode 0)."""
+def _wide_forward(L, graph, ins, W, bias, conv, training, aseed, want_out, want_planes, save_dact=False):
+    """Head-averaged output layer, aggregate-first (spgnn_gat_aggx_fwd + spgnn_wide_linear mode 0).  save_dact: also
+    keep act'(pre) of every head [N, H*F] on the tape for spgnn_wide_dpre."""
     L_ = lib()
     dev = graph.in_ptr.device
     N, E, H, F = graph.num_nodes, graph.num_edges, L.H, L.F
@@ -422,18 +429,28 @@ def _wide_forward(L, graph, ins, W, bias, conv, training, aseed, want_out, want_
     out32 = ops.empty_padded(N, F, dev) if want_out else None
     P = Planes(N, F, dev) if want_planes else None
     ws = _ws(L_.wide_linear_ws(H, F, kp, has_res), dev)
-    L_.wide_linear(XA.ptr(), XA.ld, XA.ps, kp, k_in, N, H, F, has_res, ptr(W), W.stride(0), ptr(bias), conv._act, 0,
-                   ptr(out32), out32.stride(0) if out32 is not None else 0,
-                   P.ptr() if P is not None else None, P.ld if P is not None else 0, P.ps if P is not None else 0,
-                   None, 0, None, 0, None, 0, None, 0, 0, None, ptr(ws), ws.numel(), stream(),
-                   _key=("flops", 2.0 * N * hf * k_in * (1 + has_res)))
+    outs = (ptr(out32), out32.stride(0) if out32 is not None else 0,
+            P.ptr() if P is not None else None, P.ld if P is not None else 0, P.ps if P is not None else 0)
+    flops = ("flops", 2.0 * N * hf * k_in * (1 + has_res))
+    dact = None
+    if save_dact:
+        dact = torch.empty(N, hf, dtype=torch.float32, device=dev)
+        L_.wide_linear_fwd_dact(XA.ptr(), XA.ld, XA.ps, kp, k_in, N, H, F, has_res, ptr(W), W.stride(0), ptr(bias),
+                                conv._act, *outs, ptr(dact), dact.stride(0), ptr(ws), ws.numel(), stream(),
+                                _key=flops, _name="wide_linear")
+    else:
+        L_.wide_linear(XA.ptr(), XA.ld, XA.ps, kp, k_in, N, H, F, has_res, ptr(W), W.stride(0), ptr(bias), conv._act,
+                       0, *outs, None, 0, None, 0, None, 0, None, 0, 0, None, ptr(ws), ws.numel(), stream(), _key=flops)
     rec = _WideRec()
     rec.XA, rec.att, rec.eler, rec.bias, rec.aseed, rec.kp = XA, att, eler, bias, aseed, kp
+    rec.dact = dact
     return out32, P, rec
 
 
-def _wide_backward(L, graph, rec, W, gsrcs, training, need_bias):
-    """Returns (d packed weight [ycols, k_in], d bias or None, dX fp32 [N, k_in])."""
+def _wide_backward(L, graph, rec, W, gsrcs, training, need_bias, head_grad=None):
+    """Returns (d packed weight [ycols, k_in], d bias or None, dX fp32 [N, k_in]).  head_grad: (planes of the head's
+    output gradient, head weight) when the layer output feeds the head and rec.dact was saved; the head's dX is then
+    the last gradient source, formed inside spgnn_wide_dpre."""
     L_ = lib()
     dev = graph.in_ptr.device
     N, E, H, F = graph.num_nodes, graph.num_edges, L.H, L.F
@@ -441,17 +458,27 @@ def _wide_backward(L, graph, rec, W, gsrcs, training, need_bias):
     k4 = (k_in + 3) // 4 * 4
     has_res = int(L.res_mode == 1)
     conv = L.conv
-    if not 1 <= len(gsrcs) <= 3:
+    if not 1 <= len(gsrcs) + (head_grad is not None) <= 3:
         raise SpgnnError("stack: 1..3 gradient contributions to the output layer are supported")
     XA = rec.XA
     dpre = Planes(N, hf, dev)
     db = torch.empty(hf, dtype=torch.float32, device=dev) if rec.bias is not None and need_bias else None
-    ws = _ws(L_.wide_linear_ws(H, F, kp, has_res), dev)
     gp = [(ptr(g), g.stride(0)) for g in gsrcs] + [(None, 0)] * (3 - len(gsrcs))
-    L_.wide_linear(XA.ptr(), XA.ld, XA.ps, kp, k_in, N, H, F, has_res, ptr(W), W.stride(0), ptr(rec.bias), conv._act, 1,
-                   None, 0, None, 0, 0, gp[0][0], gp[0][1], gp[1][0], gp[1][1], gp[2][0], gp[2][1],
-                   dpre.ptr(), dpre.ld, dpre.ps, ptr(db), ptr(ws), ws.numel(), stream(),
-                   _key=("flops", 2.0 * N * hf * k_in * (1 + has_res)))
+    if head_grad is not None:
+        glp, Wh = head_grad
+        Wh = ops._rows(Wh)
+        ws = _ws(L_.wide_dpre_ws(H, F), dev)
+        L_.wide_dpre(glp.ptr(), glp.ld, glp.ps, glp.cols, N, H, F, ptr(Wh), Wh.stride(0), ptr(rec.dact),
+                     rec.dact.stride(0), gp[0][0], gp[0][1], gp[1][0], gp[1][1], dpre.ptr(), dpre.ld, dpre.ps, ptr(db),
+                     ptr(ws), ws.numel(), stream(),
+                     _key=("bytes", 4.0 * N * hf * (2 + len(gsrcs) / H) + 4.0 * N * glp.cols))
+        rec.dact = None
+    else:
+        ws = _ws(L_.wide_linear_ws(H, F, kp, has_res), dev)
+        L_.wide_linear(XA.ptr(), XA.ld, XA.ps, kp, k_in, N, H, F, has_res, ptr(W), W.stride(0), ptr(rec.bias),
+                       conv._act, 1, None, 0, None, 0, 0, gp[0][0], gp[0][1], gp[1][0], gp[1][1], gp[2][0], gp[2][1],
+                       dpre.ptr(), dpre.ld, dpre.ps, ptr(db), ptr(ws), ws.numel(), stream(),
+                       _key=("flops", 2.0 * N * hf * k_in * (1 + has_res)))
     ldx = (1 + has_res) * k4
     dXA = torch.empty(H, N, ldx, dtype=torch.float32, device=dev)
     x_view = PlanesView(XA, H * kp, k_in)
@@ -520,6 +547,7 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
     d_packed, d_bias = [None] * nL, [None] * nL
     d_hw = d_hb = None
     extra = {}          # tensor -> [fp32 gradient tensors without a mask]
+    head_grad = {}      # tensor -> (head output-gradient planes, head weight): dX of the head formed by its consumer
     for name, g in g_outs.items():
         if g is not None:
             extra.setdefault(name, []).append(_grad_rows(g))
@@ -528,7 +556,11 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
         glp = split_planes(gl)
         d_hw = planes_linear_bwd_weight(glp, tape.emb_planes)
         d_hb = ops.colsum(gl)
-        extra.setdefault(plan.outputs[0], []).append(planes_linear_bwd_input(glp, head[0], head[0].shape[1]))
+        rec = tape.layers[plan.producer[plan.outputs[0]]] if plan.outputs[0] in plan.producer else None
+        if isinstance(rec, _WideRec) and rec.dact is not None and head[0].shape[0] <= 64:    # one k-block of classes
+            head_grad[plan.outputs[0]] = (glp, head[0])
+        else:
+            extra.setdefault(plan.outputs[0], []).append(planes_linear_bwd_input(glp, head[0], head[0].shape[1]))
         tape.emb_planes = None
     dX = {}             # layer index -> fp32 [N, k] gradient of its concatenated (dropped) input
     # layers whose dX already includes their own feat_drop mask: the mask is applied in the dX GEMM epilogue
@@ -545,11 +577,12 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
                 srcs.append((dX[ci], off, pm, tape.fseed[ci], (plan.layers[ci].k_in + 3) // 4))
         for g in extra.get(L.output, []):
             srcs.append((g, 0, 0.0, 0, 1))
-        if not srcs:
+        hg = head_grad.pop(L.output, None)
+        if not srcs and hg is None:
             dX[i] = None          # nothing flows into this layer: its parameters get no gradient
             tape.layers[i] = None
             continue
-        if len(srcs) > 3:
+        if len(srcs) + (hg is not None) > 3:
             raise SpgnnError("stack: more than three gradient contributions to one tensor are not supported")
         hf = L.H * L.F
         if isinstance(tape.layers[i], _WideRec):
@@ -559,7 +592,7 @@ def _backward(plan: StackPlan, graph, tape, packed, head, g_logits, g_outs, need
             if any(off for _, off, *_ in srcs):
                 raise SpgnnError("stack: a head-averaged output layer cannot take a gradient at a column offset")
             d_packed[i], d_bias[i], dX[i] = _wide_backward(L, graph, rec, packed[i], [g for g, *_ in srcs],
-                                                           tape.training, need_bias[i])
+                                                           tape.training, need_bias[i], hg)
             continue
         ins, Y, att, b = tape.layers[i]
         tape.layers[i] = None
@@ -616,13 +649,14 @@ class StackFn(Function):
     """(logits | None, *outputs) = stack(ext inputs; packed weights, biases, head) with a hand-written backward."""
 
     @staticmethod
-    def forward(ctx, plan, graph, training, ext_names, n_layers, has_head, *tensors):
+    def forward(ctx, plan, graph, training, ext_names, n_layers, has_head, grad_enabled, *tensors):
         ext = dict(zip(ext_names, tensors[:len(ext_names)]))
         o = len(ext_names)
         packed = list(tensors[o:o + n_layers])
         biases = list(tensors[o + n_layers:o + 2 * n_layers])
         head = (tensors[o + 2 * n_layers], tensors[o + 2 * n_layers + 1]) if has_head else None
-        keep = any(t is not None and t.requires_grad for t in tensors[o:])
+        # no tape when the caller runs without autograd (forward() itself always runs with grad mode off)
+        keep = grad_enabled and any(t is not None and t.requires_grad for t in tensors[o:])
         logits, outs, tape = _forward(plan, graph, ext, packed, biases, head, training, keep)
         ctx.plan, ctx.graph, ctx.tape, ctx.n_ext, ctx.n_layers, ctx.has_head = plan, graph, tape, o, n_layers, has_head
         if tape is not None:
@@ -642,11 +676,11 @@ class StackFn(Function):
         else:
             g_logits, g_outs = None, dict(zip(plan.outputs, grads))
         o = ctx.n_ext
-        need = ctx.needs_input_grad[6:]
+        need = ctx.needs_input_grad[7:]
         need_bias = [need[o + nL + i] for i in range(nL)]
         d_packed, d_bias, d_hw, d_hb = _backward(plan, ctx.graph, tape, tape.packed, tape.head, g_logits, g_outs, need_bias)
         tape.layers = None
-        out = [None] * 6 + [None] * o + d_packed + d_bias
+        out = [None] * 7 + [None] * o + d_packed + d_bias
         if ctx.has_head:
             out += [d_hw, d_hb]
         return tuple(out)
@@ -663,7 +697,8 @@ def run_stack(plan: StackPlan, graph, ext, training, head=None):
     args = [ext[n] for n in names] + packed + biases
     if head is not None:
         args += [head.weight, head.bias]
-    res = StackFn.apply(plan, graph, bool(training), tuple(names), len(plan.layers), head is not None, *args)
+    res = StackFn.apply(plan, graph, bool(training), tuple(names), len(plan.layers), head is not None,
+                        torch.is_grad_enabled(), *args)
     if head is not None:
         return res[0], list(res[1:])
     return None, list(res)
