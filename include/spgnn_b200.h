@@ -122,7 +122,7 @@ int spgnn_linear_bwd_weight2(const float* dC, int64_t lddc, const float* A1, int
 /* ------------------------------------------------------------------------------------
  * Dense projection over "planes" operands — the production path of the same DGL projections (GATConv.fc / res_fc,
  * gnn_out; models.py:301-314, 425-456, 1167-1170).
- * Planes: an fp32-valued matrix X[rows, cols] stored as TWO bf16 matrices, X = hi + lo (|residual| <= 2^-18 |X|),
+ * Planes: an fp32-valued matrix X[rows, cols] stored as TWO bf16 matrices, X = hi + lo (|residual| <= 2^-17 |X|),
  * both [rows, ld] row-major; the pointer passed is `hi`, lo = hi + plane_stride (elements).  ld and plane_stride must
  * be multiples of 8 (16-byte rows), the base 16-byte aligned.  Same bytes as fp32, but the tensor cores consume them
  * directly: operands go global -> shared by TMA and every product is hi*hi + hi*lo + lo*hi with fp32 accumulation

@@ -1,6 +1,6 @@
 // tcgen05 tensor-core GEMMs for the dense projections (mode 1), fp32 in / fp32 out, fp32-grade accuracy.
 //
-// Arithmetic: every fp32 operand is split into two bf16 terms, a = a_hi + a_lo (|residual| <= 2^-18 |a|), and the
+// Arithmetic: every fp32 operand is split into two bf16 terms, a = a_hi + a_lo (|residual| <= 2^-17 |a|), and the
 // product is formed as  a_hi*b_hi + a_hi*b_lo + a_lo*b_hi  with fp32 accumulation in TMEM ("bf16x3"): three
 // kind::f16 UMMAs per k-step, relative error ~3*2^-18 per product — inside the 1e-4 parity bar with margin, at 3/2 of
 // the cost of ONE tf32 pass (a single tf32 pass would break parity; 3xTF32 would cost twice this).

@@ -1,6 +1,6 @@
 // TMA-fed tcgen05 GEMMs over "planes" operands (the production projection path).
 //
-// Planes: an fp32-valued matrix X[rows, cols] held as TWO bf16 matrices, X = hi + lo (|residual| <= 2^-18 |X|),
+// Planes: an fp32-valued matrix X[rows, cols] held as TWO bf16 matrices, X = hi + lo (|residual| <= 2^-17 |X|),
 // both [rows, ld] row-major, lo = hi + plane_stride.  Same bytes as fp32, but directly consumable by the tensor
 // cores: the product a*b is formed as a_hi*b_hi + a_hi*b_lo + a_lo*b_hi with fp32 accumulation in TMEM (three
 // kind::f16 UMMAs per k-step, relative error ~3*2^-18 per product — inside the 1e-4 parity bar, see gemm_tc.cu).

@@ -173,7 +173,8 @@ __host__ __device__ __forceinline__ uint32_t make_idesc_pair(int n) {
 }
 
 // fp32 pair -> packed bf16 (hi) and packed bf16 of the remainders (lo); low half = first element.
-// a = hi + lo + r with |r| <= 2^-18 |a|.
+// a = hi + lo + r with |r| <= 2^-17 |a| for normal a (the largest over all 2^23 mantissas of a binade is
+// 2^-17.003: each rounding keeps 8 significant bits, the two together 16 and a sign).
 __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
     __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
     hi = *reinterpret_cast<uint32_t*>(&h);

@@ -95,6 +95,26 @@ def oracle_fp64(onet, og):
     return net64, g64
 
 
+def launches(run):
+    """Short names of the library kernels run() launches, template arguments included ('spmm_kernel<4>',
+    'act_bwd_planes_kernel<true>'); torch's own kernels are left out.  A throwaway kernel opens the profiler session:
+    the profiler has been seen to drop the first launch of a session."""
+    import re
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        torch.ones(1, device="cuda").add_(1)
+        torch.cuda.synchronize()
+        run()
+        torch.cuda.synchronize()
+    names = set()
+    for e in prof.events():
+        if "spgnn::" not in e.name:
+            continue
+        m = re.search(r"(\w+_kernel)\s*(<[\w,\s]*>)?\s*\(", e.name)
+        if m:
+            names.add(m.group(1) + re.sub(r"\s+", "", m.group(2) or ""))
+    return names
+
+
 def traced(ops, fn):
     """Runs fn() on the device with spgnn_b200.ops.KINK_TRACE recording; returns (result, records)."""
     ops.KINK_TRACE = []
