@@ -538,6 +538,36 @@ int spgnn_edges_expand(const int32_t* src32, const int32_t* dst32, const int64_t
                        void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Neighbour-sampled blocks for SAGE mini-batches (DGL MultiLayerNeighborSampler + to_block + the block CSC/CSR;
+ * job_runner.py:1460-1514 via sampling.DeviceBlockSampler).  All L layers in one launch of one CTA, stream-ordered.
+ *   graph    : in_ptr int32 [N+1], in_src int32 (in-CSC, ascending edge id per destination)
+ *   seeds    : int64 [S] distinct node ids in [0, N) (checked on the device as well)
+ *   per layer l (0 = input layer; the output layer L-1 is drawn first, its destinations are the seeds and every
+ *   layer's destinations are the next layer's sources):
+ *     fanouts_host[l]      : edges kept per destination, min(fanout, in-degree), uniformly without replacement;
+ *                            -1 keeps all.  Key of CSC slot s: mix64(mix64(seed ^ mix64(salt ^ (l+1) << 56)) ^ s);
+ *                            the `fanout` smallest (key, slot) pairs are kept, emitted in ascending slot order.
+ *     caps_host[3l..3l+2]  : capacities {destinations, sources, edges} of the buffers below
+ *     bufs_host[6l..6l+5]  : device addresses of in_ptr int32 [cap_dst+1], in_src int32 [cap_e] (local source ids),
+ *                            out_ptr int32 [cap_src+1], out_dst int32 [cap_e], out_slot int32 [cap_e] (stable by
+ *                            source; out_slot = position in the in-CSC), src_ids int64 [cap_src] (the destinations,
+ *                            then every other source once in ascending id)
+ *   pos      : int32 [N], all -1 on entry and on return (the call resets what it sets)
+ *   edst_ws  : int32 [edst_cap >= largest cap_e]; keys_ws: uint64 [keys_cap], a power of two >= every cap_e and
+ *              cap_src - cap_dst that exceeds 4096 (0 / null when none does)
+ *   sizes    : int64 [2L+1]: (num_src, num_edges) of layer l at 2l, 2l+1; sizes[2L] = 0, or the error code when a
+ *              capacity was too small (1), a seed was out of range (2) or repeated (3), in_src held a bad id (4).
+ *              The caller reads it before trusting anything else.
+ * gather_rows: out[r, :] = x[idx[r], :] in 32-bit words for r < min(cap, *count) (count null: r < cap); rows whose
+ *              idx is outside [0, n_rows) are skipped. */
+int spgnn_sample_blocks(const int32_t* in_ptr, const int32_t* in_src, int64_t N, const int64_t* seeds, int64_t S,
+                        int64_t L, const int64_t* fanouts_host, const int64_t* caps_host, const int64_t* bufs_host,
+                        uint64_t seed, uint64_t salt, int32_t* pos, int32_t* edst_ws, int64_t edst_cap,
+                        uint64_t* keys_ws, int64_t keys_cap, int64_t* sizes, void* stream);
+int spgnn_gather_rows(const void* x, int64_t ldx_words, int64_t n_rows, const int64_t* idx, const int64_t* count,
+                      int64_t cap, int64_t words, void* out, int64_t ldo_words, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Synthetic airway trees on device (bench input; integer part bit-identical to spgnn_b200/synth.py).
  * ---------------------------------------------------------------------------------- */
 int spgnn_synth_trees(int64_t first_tree, int64_t B, uint32_t seed, int ragged, int64_t k_fixed,

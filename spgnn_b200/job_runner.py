@@ -282,20 +282,22 @@ class GCNTrainSPGNN(GCNTrain):
 class GCNTrainSAGE(GCNTrain):
     """GCNTrainSAGE.train (job_runner.py:1460-1514): every GCN step draws ``node_sample_rate`` of the batch's nodes,
     walks them in mini-batches of NODE_BATCH_SIZE seeds through ``MultiLayerNeighborSampler(node_ks)`` blocks and
-    takes one optimiser step per mini-batch with the class-weighted CE over the seeds (no node mask here)."""
+    takes one optimiser step per mini-batch with the class-weighted CE over the seeds (no node mask here).  The
+    blocks come from ``sampling.DeviceBlockSampler``: the same distribution as DGL's sampler, drawn from the
+    counter hash of the dropout masks (seeded by ``ops.manual_seed``) instead of torch's generator."""
 
     def train_batch(self, scans, steps=None, max_minibatches=None):
         from . import sampling
         s = self.settings
         self.model.train()
         g = self.to_device(scans)
-        sampler = sampling.MultiLayerNeighborSampler(self.model.sage.node_ks)
+        sampler = sampling.DeviceBlockSampler(self.model.sage.node_ks)
         node_bs = int(getattr(s, "NODE_BATCH_SIZE", 64))
         losses = []
         for n in range(s.GCN_STEPS if steps is None else steps):
             nids = random.sample(range(g.num_nodes), int(g.num_nodes * self.model.sage.node_sample_rate))
-            loader = sampling.NodeDataLoader(g, nids, sampler, device=self.device, batch_size=node_bs, shuffle=True,
-                                             drop_last=False)
+            loader = sampling.DeviceNodeDataLoader(g, nids, sampler, device=self.device, batch_size=node_bs,
+                                                   shuffle=True, drop_last=False)
             loss = None
             for k, (input_nodes, seeds, blocks) in enumerate(loader):
                 if max_minibatches is not None and k >= max_minibatches:
