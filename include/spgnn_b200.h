@@ -89,39 +89,9 @@ int spgnn_batch_build(const int64_t* node_off, const int64_t* edge_off, int64_t 
                       int32_t* flags, void* ws, void* stream);
 
 /* ------------------------------------------------------------------------------------
- * Dense projection (DGL GATConv.fc / res_fc, GraphConv weight, SAGEConv fc_*, GIN MLP, gnn_out):
- * SURVEY §2.1 K1/K8.  fp32 in, fp32 out.
- *   C[M,N] (ldc) = [A1 | A2][M,K1+K2] * W[N, K1+K2 (ldw)]^T  (+ bias[N]) (act)
- * A2 may be null (K2 = 0): the two-source form removes torch.cat([h_s,h_p]) (models.py:477,481).
- * mode: 0 = fp32 SIMT, 1 = tcgen05 tensor cores with split-bf16 operands (a = hi + lo; hi*hi + hi*lo + lo*hi,
- *       fp32 accumulate in TMEM; relative error ~1e-5) — falls back to mode 0 when 16-byte alignment of the
- *       operands / leading dimensions is not given.  ws: scratch for the pre-split weight, spgnn_linear_fwd_ws /
- *       spgnn_linear_bwd_input_ws bytes (mode 1 only).
- * ---------------------------------------------------------------------------------- */
-int64_t spgnn_linear_fwd_ws(int64_t N, int64_t K1, int64_t K2);
-int spgnn_linear_fwd(const float* A1, int64_t lda1, int64_t K1, const float* A2, int64_t lda2, int64_t K2,
-                     const float* W, int64_t ldw, const float* bias, int act, float slope,
-                     float* C, int64_t ldc, int64_t M, int64_t N, int mode, void* ws, int64_t ws_bytes, void* stream);
-/* dA[M,K] (ldda) = dC[M,N] (lddc) * W[N, k_off : k_off+K] (ldw) */
-int64_t spgnn_linear_bwd_input_ws(int64_t N, int64_t K);
-int spgnn_linear_bwd_input(const float* dC, int64_t lddc, const float* W, int64_t ldw, int64_t k_off,
-                           float* dA, int64_t ldda, int64_t M, int64_t N, int64_t K, int mode,
-                           void* ws, int64_t ws_bytes, void* stream);
-/* dW[N, k_off : k_off+K] (lddw) = dC[M,N]^T * A[M,K] (lda); split over M into `splits` partial sums in ws
- * (splits*N*K floats, see spgnn_linear_bwd_weight_ws) that a second kernel reduces deterministically. */
-int64_t spgnn_linear_bwd_weight_ws(int64_t M, int64_t N, int64_t K);
-int spgnn_linear_bwd_weight(const float* dC, int64_t lddc, const float* A, int64_t lda,
-                            float* dW, int64_t lddw, int64_t k_off, int64_t M, int64_t N, int64_t K,
-                            void* ws, int mode, void* stream);
-/* Two-source form: dW[N, K1+K2] (lddw) = dC[M,N]^T * [A1 | A2] in ONE pass over dC (mode 1: 256 x BN tensor-core tiles
- * with two TMEM accumulators sharing the dC tile). */
-int64_t spgnn_linear_bwd_weight2_ws(int64_t M, int64_t N, int64_t K1, int64_t K2);
-int spgnn_linear_bwd_weight2(const float* dC, int64_t lddc, const float* A1, int64_t lda1, int64_t K1,
-                             const float* A2, int64_t lda2, int64_t K2, float* dW, int64_t lddw,
-                             int64_t M, int64_t N, void* ws, int mode, void* stream);
-/* ------------------------------------------------------------------------------------
- * Dense projection over "planes" operands — the production path of the same DGL projections (GATConv.fc / res_fc,
- * gnn_out; models.py:301-314, 425-456, 1167-1170).
+ * Dense projection over "planes" operands (DGL GATConv.fc / res_fc, GraphConv weight, SAGEConv fc_*, GIN MLP,
+ * gnn_out; models.py:301-314, 425-456, 1167-1170; SURVEY §2.1 K1/K8).  A2 may be null (K2 = 0): the two-source form
+ * removes torch.cat([h_s,h_p]) (models.py:477,481).
  * Planes: an fp32-valued matrix X[rows, cols] stored as TWO bf16 matrices, X = hi + lo (|residual| <= 2^-17 |X|),
  * both [rows, ld] row-major; the pointer passed is `hi`, lo = hi + plane_stride (elements).  ld and plane_stride must
  * be multiples of 8 (16-byte rows), the base 16-byte aligned.  Same bytes as fp32, but the tensor cores consume them

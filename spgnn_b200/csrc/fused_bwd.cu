@@ -2,6 +2,7 @@
 //   d = mask(g) * act'(y)   ->   split-bf16 planes of d (the operand of the dX / dW GEMMs)  +  column sums of d (bias gradient)
 // instead of act_bwd (read g, y; write d), split_planes (read d; write planes) and colsum (read d): 12 bytes per
 // element instead of 28.  HBM-bound; one warp per row segment of 128 columns, float4 per lane.
+// spgnn_colsum is the column sum alone, for the bias gradients of the paths that do not go through that pass.
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -82,9 +83,54 @@ __global__ void sum_bands_kernel(const float* __restrict__ part, int64_t bands, 
 }
 
 }  // namespace
+
+// column sums: partial per block over a row band, then a fixed-order final reduce
+__global__ void colsum_partial_kernel(const float* __restrict__ X, int64_t ldx, int64_t M, int64_t N,
+                                      int64_t rows_per_block, float* __restrict__ part) {
+    const int64_t r0 = (int64_t)blockIdx.y * rows_per_block;
+    const int64_t r1 = r0 + rows_per_block < M ? r0 + rows_per_block : M;
+    for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < N; c += (int64_t)gridDim.x * blockDim.x) {
+        float s = 0.f;
+        for (int64_t r = r0; r < r1; ++r) s += __ldg(X + r * ldx + c);
+        part[(int64_t)blockIdx.y * N + c] = s;
+    }
+}
+// one warp per column: lane l adds the partial rows l, l + 32, ... then a butterfly (a fixed order, hence reproducible);
+// one thread per column walked 592 dependent loads: 50 us for the 22 columns of the head's bias gradient
+__global__ void colsum_final_kernel(const float* __restrict__ part, int64_t nparts, int64_t N, float* __restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t c = warp; c < N; c += nwarps) {
+        float s = 0.f;
+        for (int64_t p = lane; p < nparts; p += 32) s += part[p * N + c];
+        s = warp_sum(s);
+        if (lane == 0) out[c] = s;
+    }
+}
+
+constexpr int64_t kColsumParts = 592;   // 4 x 148 row bands
+
 }  // namespace spgnn
 
 using namespace spgnn;
+
+extern "C" int64_t spgnn_colsum_ws(int64_t N) { return kColsumParts * N * (int64_t)sizeof(float); }
+
+extern "C" int spgnn_colsum(const float* X, int64_t ldx, int64_t M, int64_t N, float* out, void* ws, void* stream) {
+    SPGNN_REQUIRE(X && out && ws && M > 0 && N > 0, "colsum: bad argument");
+    cudaStream_t st = as_stream(stream);
+    int64_t parts = M < kColsumParts ? M : kColsumParts;
+    int64_t rpb = ceil_div(M, parts);
+    parts = ceil_div(M, rpb);
+    dim3 grid((unsigned)ceil_div(N, 128), (unsigned)parts);
+    colsum_partial_kernel<<<grid, 128, 0, st>>>(X, ldx, M, N, rpb, (float*)ws);
+    SPGNN_LAUNCH_OK();
+    const int64_t fblocks = ceil_div(N * 32, 128), fcap = (int64_t)sm_count() * 8;
+    colsum_final_kernel<<<(unsigned)(fblocks < fcap ? fblocks : fcap), 128, 0, st>>>((const float*)ws, parts, N, out);
+    SPGNN_LAUNCH_OK();
+    return SPGNN_OK;
+}
 
 extern "C" int64_t spgnn_act_bwd_planes_ws(int64_t N) { return kFbMaxBands * N * (int64_t)sizeof(float) + 16; }
 

@@ -3,7 +3,8 @@
 // Planes: an fp32-valued matrix X[rows, cols] held as TWO bf16 matrices, X = hi + lo (|residual| <= 2^-17 |X|),
 // both [rows, ld] row-major, lo = hi + plane_stride.  Same bytes as fp32, but directly consumable by the tensor
 // cores: the product a*b is formed as a_hi*b_hi + a_hi*b_lo + a_lo*b_hi with fp32 accumulation in TMEM (three
-// kind::f16 UMMAs per k-step, relative error ~3*2^-18 per product — inside the 1e-4 parity bar, see gemm_tc.cu).
+// kind::f16 UMMAs per k-step, relative error ~3*2^-18 per product — inside the 1e-4 parity bar with margin, at 3/2 of
+// the cost of ONE tf32 pass; a single tf32 pass would break that bar).
 // The kernels that PRODUCE activations (aggregation epilogues, spgnn_split_planes) write planes, so no GEMM converts
 // anything: operands go global -> shared by TMA (cp.async.bulk.tensor, SWIZZLE_128B) and shared -> tensor core by
 // UMMA descriptors; no register staging, several stages (64-96 KB each) in flight per SM.
@@ -1296,8 +1297,29 @@ using namespace spgnn;
 using namespace spgnn::tma;
 
 namespace spgnn {
-void reduce_splits(const float* ws, int64_t splits, int64_t N, int64_t K, float* out, int64_t ldo, cudaStream_t st);
+__global__ void reduce_splits_kernel(const float* __restrict__ ws, int64_t splits, int64_t split_stride, int64_t N,
+                                     int64_t K, float* __restrict__ out, int64_t ldo) {
+    const int64_t total = N * K;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        // fixed order: eight interleaved running sums (independent loads in flight), combined pairwise at the end
+        float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        int64_t z = 0;
+        for (; z + 8 <= splits; z += 8) {
+#pragma unroll
+            for (int u = 0; u < 8; ++u) s[u] += __ldg(ws + (z + u) * split_stride + i);
+        }
+        for (int u = 0; z < splits; ++z, ++u) s[u] += __ldg(ws + z * split_stride + i);
+        out[(i / K) * ldo + (i % K)] = ((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]));
+    }
 }
+
+void reduce_splits(const float* ws, int64_t splits, int64_t N, int64_t K, float* out, int64_t ldo, cudaStream_t st) {
+    const int64_t total = N * K;
+    const int64_t want = ceil_div(total, 256), cap = (int64_t)sm_count() * 8;
+    reduce_splits_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(ws, splits, N * K, N, K, out, ldo);
+    count_launch();
+}
+}  // namespace spgnn
 
 extern "C" int spgnn_split_planes(const float* x1, int64_t ld1, int64_t K1, const float* x2, int64_t ld2, int64_t K2,
                                   float p, uint64_t seed, int64_t concat_chunks, int64_t chunk_off, uint16_t* out_hi,

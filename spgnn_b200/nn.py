@@ -279,7 +279,7 @@ class GINConv(nn.Module):
         mlp = self.apply_func
         if mlp is None:
             return rst
-        if ops.GEMM_MODE == 2 and _is_gin_mlp(mlp) and rst.is_cuda:
+        if _is_gin_mlp(mlp) and rst.is_cuda:
             # the reference's MLP in one Function: no dropout pass in either direction (ops.MlpDropFn)
             return ops.mlp_drop(rst, mlp[0].weight, mlp[0].bias, mlp[3].weight, mlp[3].bias, "leaky_relu",
                                 mlp[0]._slope, mlp[1].p if mlp[1].training else 0.0)

@@ -12,9 +12,9 @@ from ._lib import SpgnnError, lib, ptr, require_cuda, stream
 
 ACT = {None: 0, "none": 0, "elu": 1, "tanh": 2, "relu": 3, "leaky_relu": 4}
 
-# projection arithmetic of ``linear`` (GraphConv / SAGEConv / GINConv / nn.Linear; GAT stacks always take the planes
-# pipeline of stack.py): 0 = fp32 SIMT, 1 = tcgen05 split-bf16 with in-kernel conversion (csrc/gemm_tc.cu),
-# 2 = planes + TMA-fed tcgen05 (csrc/gemm_tma.cu)
+# The one projection arithmetic: the planes + TMA-fed tcgen05 GEMMs of csrc/gemm_tma.cu, behind ``linear``, the GIN
+# MLP, the LSTM reducer and the GAT stacks alike.  bench.py sets GEMM_MODE from --gemm-mode and writes it into its JSON
+# line; stack.planes_linear refuses any value but 2, so no run is reported under a mode it did not use.
 GEMM_MODE = 2
 
 # Test hook (oracle/kinks.py replays it): when a list, every non-smooth decision the path takes is appended in call
@@ -103,68 +103,6 @@ def colsum(x):
     return out
 
 
-class LinearFn(Function):
-    """y = act([x1 | x2] @ W^T + bias).  W is [N, K1+K2] with unit inner stride (any row stride)."""
-
-    @staticmethod
-    def forward(ctx, x1, x2, W, bias, act, slope):
-        require_cuda(x1, x2, W, bias)
-        x1 = _rows(x1)
-        x2 = _rows(x2) if x2 is not None else None
-        W = _rows(W)
-        M, K1 = x1.shape
-        K2 = x2.shape[1] if x2 is not None else 0
-        N = W.shape[0]
-        if W.shape[1] != K1 + K2:
-            raise SpgnnError(f"linear: weight has {W.shape[1]} columns, input has {K1}+{K2}")
-        y = empty_padded(M, N, x1.device)
-        b = bias.contiguous() if bias is not None else None
-        ws = _ws(lib().linear_fwd_ws(N, K1, K2), x1.device) if GEMM_MODE == 1 else None
-        lib().linear_fwd(ptr(x1), x1.stride(0), K1, ptr(x2), x2.stride(0) if x2 is not None else 0, K2,
-                         ptr(W), W.stride(0), ptr(b), act, float(slope), ptr(y), y.stride(0), M, N, GEMM_MODE,
-                         ptr(ws), ws.numel() if ws is not None else 0, stream(),
-                         _key=("flops", 2.0 * M * N * (K1 + K2)))
-        ctx.save_for_backward(x1, x2, W, y if act else None)
-        ctx.cfg = (act, float(slope), bias is not None)
-        return y
-
-    @staticmethod
-    def backward(ctx, g):
-        x1, x2, W, y = ctx.saved_tensors
-        act, slope, has_bias = ctx.cfg
-        L = lib()
-        g = _rows(g)
-        M, N = g.shape
-        K1 = x1.shape[1]
-        K2 = x2.shape[1] if x2 is not None else 0
-        if act:
-            d = empty_padded(M, N, g.device)
-            L.act_bwd(ptr(g), g.stride(0), ptr(y), y.stride(0), act, slope, ptr(d), d.stride(0), M, N, stream())
-            g = d
-        dx1 = dx2 = dW = db = None
-        if ctx.needs_input_grad[0]:
-            dx1 = empty_padded(M, K1, g.device)
-            ws = _ws(L.linear_bwd_input_ws(N, K1), g.device) if GEMM_MODE == 1 else None
-            L.linear_bwd_input(ptr(g), g.stride(0), ptr(W), W.stride(0), 0, ptr(dx1), dx1.stride(0), M, N, K1,
-                               GEMM_MODE, ptr(ws), ws.numel() if ws is not None else 0, stream(),
-                               _key=("flops", 2.0 * M * N * K1))
-        if x2 is not None and ctx.needs_input_grad[1]:
-            dx2 = empty_padded(M, K2, g.device)
-            ws = _ws(L.linear_bwd_input_ws(N, K2), g.device) if GEMM_MODE == 1 else None
-            L.linear_bwd_input(ptr(g), g.stride(0), ptr(W), W.stride(0), K1, ptr(dx2), dx2.stride(0), M, N, K2,
-                               GEMM_MODE, ptr(ws), ws.numel() if ws is not None else 0, stream(),
-                               _key=("flops", 2.0 * M * N * K2))
-        if ctx.needs_input_grad[2]:
-            dW = empty_padded(N, K1 + K2, g.device)
-            ws = _ws(L.linear_bwd_weight2_ws(M, N, K1, K2), g.device)
-            L.linear_bwd_weight2(ptr(g), g.stride(0), ptr(x1), x1.stride(0), K1, ptr(x2),
-                                 x2.stride(0) if x2 is not None else 0, K2, ptr(dW), dW.stride(0), M, N, ptr(ws),
-                                 GEMM_MODE, stream(), _key=("flops", 2.0 * M * N * (K1 + K2)))
-        if has_bias and ctx.needs_input_grad[3]:
-            db = colsum(g)
-        return dx1, dx2, dW, db, None, None
-
-
 def _planes_of(x):
     """Planes of an fp32 activation, converted once per tensor: a tensor feeding several projections (SAGEConv's
     ``h`` goes to fc_pool and fc_self) is split a single time.  The planes ride on the tensor object and are
@@ -182,7 +120,7 @@ def _planes_of(x):
 
 
 class PlanesLinearFn(Function):
-    """y = act([x1 | x2] @ W^T + bias) through the planes pipeline (GEMM_MODE 2): the inputs are converted to
+    """y = act([x1 | x2] @ W^T + bias) through the planes pipeline: the inputs are converted to
     split-bf16 planes once (``spgnn_split_planes``), the projection and both of its gradients are the TMA-fed
     tcgen05 GEMMs of csrc/gemm_tma.cu, and the backward keeps the input PLANES (same bytes as the fp32 input)."""
 
@@ -313,10 +251,7 @@ def mlp_drop(x, W0, b0, W3, b3, act="leaky_relu", slope=0.01, p=0.0):
 
 def linear(x1, W, bias=None, act=None, slope=0.0, x2=None):
     code = act_code(act)
-    if GEMM_MODE == 2:
-        out = PlanesLinearFn.apply(x1, x2, W, bias, code, slope)
-    else:
-        out = LinearFn.apply(x1, x2, W, bias, code, slope)
+    out = PlanesLinearFn.apply(x1, x2, W, bias, code, slope)
     if tracing() and code in (ACT["relu"], ACT["leaky_relu"]):
         trace("sign", out > 0)          # the activation is fused; sign(out) == sign(pre-activation)
     return out
@@ -589,7 +524,7 @@ class LstmReduceFn(Function):
     (``linear``: autograd takes its gradients), ``W_hh`` [4D, D].  Returns [n_dst, D]; zero for in-degree 0.
 
     Step t runs over the first n_t rows of ``LstmOrder`` (destinations by descending in-degree); step 0 needs no
-    GEMM (h_0 = 0), step t ≥ 1 adds R_t = H_{t-1}[:n_t]·W_hhᵀ from the planes GEMMs whatever ``GEMM_MODE`` says.
+    GEMM (h_0 = 0), step t ≥ 1 adds R_t = H_{t-1}[:n_t]·W_hhᵀ from the planes GEMMs.
     Per-step buffers hold step t at rows [off_t, off_t + n_t): the gate activations (as the 16-bit halves of the
     planes the backward overwrites with the gate gradients), c, and h as planes at the rows of the step that reads
     it, so dW_hh is ONE GEMM over all steps."""

@@ -159,6 +159,8 @@ def _ws(nbytes, device):
 def planes_linear(A1: Planes, W, bias=None, act=0, slope=0.0, A2: Planes | None = None, out=None):
     """fp32 [M, N] = [A1 | A2] @ W^T (+bias)(act); W fp32 [N, K1+K2] with unit inner stride.  ``out``: an [M, N]
     destination with 16-byte aligned rows (a buffer reused across calls)."""
+    if ops.GEMM_MODE != 2:
+        raise SpgnnError(f"ops.GEMM_MODE = {ops.GEMM_MODE!r}: the planes GEMMs (2) are the only projection path")
     W = ops._rows(W)
     M, N = A1.rows, W.shape[0]
     K1, K2 = A1.cols, (A2.cols if A2 is not None else 0)

@@ -130,7 +130,7 @@ def test_batch_builder_csc_csr_consistency_ragged_64(mods):
                        torch.repeat_interleave(torch.arange(64), g.batch_num_nodes().cpu()))
 
 
-def test_graph_errors(mods):
+def test_graph_errors(mods, monkeypatch):
     sg = mods["sg"]
     from spgnn_b200._lib import SpgnnError
     g = sg.from_edges([0, 1], [1, 2], 3)                     # node 0 has no in-edge
@@ -141,20 +141,19 @@ def test_graph_errors(mods):
         sg.from_edges([0, 5], [1, 2], 3)                     # endpoint outside the graph
     with pytest.raises(SpgnnError):
         mods["ops"].linear(torch.zeros(4, 4), torch.zeros(4, 4))   # CPU tensors: no fallback
+    monkeypatch.setattr(mods["ops"], "GEMM_MODE", 1)                 # no projection path but the planes GEMMs
+    with pytest.raises(SpgnnError):
+        mods["ops"].linear(torch.zeros(4, 4, device="cuda"), torch.zeros(4, 4, device="cuda"))
 
 
 # ------------------------------------------------------------------------------------------------ projection
-@pytest.mark.parametrize("mode", [0, 1, 2])
 @pytest.mark.parametrize("M,K1,K2,N", [(300, 64, 0, 48), (1000, 1024, 39, 130), (257, 39, 0, 258), (513, 100, 7, 22),
                                        (128, 64, 0, 16), (5000, 1024, 40, 1028), (4096, 192, 0, 4100),
                                        (64, 64, 0, 24), (10, 1024, 0, 256), (1, 128, 128, 64)])   # mini-batch sized
-def test_linear_fwd_bwd_against_fp64(mods, M, K1, K2, N, mode, monkeypatch):
-    """mode 0: fp32 SIMT kernels; mode 1: tcgen05 split-bf16 tensor-core kernels with in-kernel conversion (falls
-    back per call when an operand is not 16-byte aligned); mode 2 (the default): planes + TMA-fed tcgen05 GEMMs.
-    All against an fp64 reference."""
+def test_linear_fwd_bwd_against_fp64(mods, M, K1, K2, N):
+    """ops.linear (planes + TMA-fed tcgen05 GEMMs) forward and backward against an fp64 reference."""
     ops = mods["ops"]
-    monkeypatch.setattr(ops, "GEMM_MODE", mode)
-    tol = 1e-5 if mode == 0 else 4e-5
+    tol = 4e-5
     gen = torch.Generator().manual_seed(M + N)
     x1 = torch.randn(M, K1, generator=gen)
     x2 = torch.randn(M, K2, generator=gen) if K2 else None
@@ -207,20 +206,13 @@ def _margin_aware_flips(a, b, tol):
     return int((margin[flips] > tol).sum())
 
 
-def _full_cases():
-    out = []
-    for name in sorted(FULL_MODELS):
-        out.append((name, 2))                       # planes + TMA-fed tensor-core projections (the default)
-        if FULL_MODELS[name][0] in ("gin", "sage", "gcn"):
-            out.append((name, 1))                   # tensor cores with in-kernel conversion
-            out.append((name, 0))                   # fp32 SIMT projections
-    return out
-
-
-@pytest.mark.parametrize("name,mode", _full_cases())
-def test_full_width_forward_backward_vs_oracle(mods, name, mode, monkeypatch):
-    """exp_settings widths, 6 ragged trees, eval-mode forward + all parameter gradients vs the CPU oracle, in every
-    GEMM mode and at the SAME bar (1e-4 outputs, 2e-4 gradients) for every model family.
+# every model, and GIN once more with its MLP run module by module (Linear, Dropout, fused LeakyReLU, Linear): the
+# branch of nn.GINConv.forward that any apply_func other than the reference's MLP takes
+@pytest.mark.parametrize("name,unfused", [pytest.param(n, False, id=n) for n in sorted(FULL_MODELS)] +
+                         [pytest.param("st_gin_3", True, id="st_gin_3-unfused")])
+def test_full_width_forward_backward_vs_oracle(mods, name, unfused, monkeypatch):
+    """exp_settings widths, 6 ragged trees, eval-mode forward + all parameter gradients vs the CPU oracle, at the
+    SAME bar (1e-4 outputs, 2e-4 gradients) for every model family.
 
     The gradient of a LeakyReLU / ReLU / max is a discontinuous function of the forward values: an attention logit,
     an MLP pre-activation or a pair of pooled neighbours within rounding distance of the kink / the tie takes one
@@ -232,7 +224,9 @@ def test_full_width_forward_backward_vs_oracle(mods, name, mode, monkeypatch):
     exactly."""
     kind, cfg = FULL_MODELS[name]
     ops = mods["ops"]
-    monkeypatch.setattr(ops, "GEMM_MODE", mode)
+    if unfused:
+        from spgnn_b200 import nn as snn
+        monkeypatch.setattr(snn, "_is_gin_mlp", lambda mlp: False)
     scans = _scan_dicts(mods, 1000, 6, ragged=True)
     pos = None
     if kind == "spgnn":
@@ -277,7 +271,7 @@ def test_full_width_forward_backward_vs_oracle(mods, name, mode, monkeypatch):
     dec = ops.segmented_argmax(out[0].detach(), g).cpu()
     dec_ref = mods["om"].decide_per_tree(ref[0].detach(), og.batch_num_nodes())
     assert torch.equal(dec, dec_ref)
-    assert_grads_match(net, onet64, GRAD_TOL, (name, mode, f"{tape.flips} of {tape.decisions} decisions pinned"))
+    assert_grads_match(net, onet64, GRAD_TOL, (name, unfused, f"{tape.flips} of {tape.decisions} decisions pinned"))
 
 
 @pytest.mark.parametrize("name", ["st_gat_3", "st_gat_6_nr", "st_pgat_spgnn_3", "st_pgat_spgnnnl_3"])
